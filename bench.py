@@ -3,6 +3,8 @@
 
   python bench.py --gpus N --steps K --warmup W            our arm (libicdrag.so on B200)
   python bench.py --impl reference --gpus N --steps K ...  the reference's CPU path (oracle port)
+  python bench.py ... --dump-outputs DIR                    also write the last timed step's results as DIR/*.npy, so
+                                                            two builds can be compared output for output (same inputs)
 
 Workload (config.workload): exact top-10 inner-product search of a batch of 1024 synthetic
 768-d bf16 queries over a synthetic 100 M x 768 bf16 corpus -- BASELINE.json configs[4].  The
@@ -42,6 +44,7 @@ if ROOT not in sys.path:
 DIM = 768
 K_TOP = 10
 PKG = "rag-project-icd10_b200"
+DUMP_MAX_BYTES = 64 << 20
 
 
 def _peaks():
@@ -63,6 +66,25 @@ def _ncu_traffic(key):
         return (ent["bytes"], ent["capture"]) if ent else (None, None)
     except Exception:
         return None, None
+
+
+def dump_outputs(out_dir, score, raw, ids):
+    """--dump-outputs: what search() hands its caller for the headline batch -- level-weighted scores, raw inner
+    products and global row ids, [B, k] each -- as out_dir/<name>.npy in float32 / float64 (ids are exact in float64).
+    Above DUMP_MAX_BYTES in all, a fixed seeded sample of query rows is written, its row numbers in query_rows.npy."""
+    import numpy as np
+    import torch
+    arrays = {"scores": score.float(), "raw_scores": raw.float(), "ids": ids.double()}
+    n = score.shape[0]
+    row_bytes = sum(a.element_size() * a.shape[1] for a in arrays.values())
+    if n * row_bytes > DUMP_MAX_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_BYTES // (row_bytes + 8), replace=False))
+        sel = torch.from_numpy(rows).to(score.device)
+        arrays = {name: a[sel] for name, a in arrays.items()}
+        arrays["query_rows"] = torch.from_numpy(rows.astype(np.float64))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
 
 
 def _icd_env():
@@ -669,7 +691,13 @@ def main():
     ap.add_argument("--no-encoder", action="store_true")
     ap.add_argument("--no-points", action="store_true", help="skip the hbm_point / ridge_point measurements")
     ap.add_argument("--no-text", action="store_true", help="skip the encoder's text-in e2e")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the headline search results of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU arm's results (--impl ours)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -789,6 +817,7 @@ def main():
             step_device()
         e1.record(stream)
         barrier()
+        last = tuple(t.clone() for t in o)     # results of the last timed step (the untimed steps below rewrite o)
         ms_total = e0.elapsed_time(e1)
         launches = native.lib().icd_launch_count() - launches0
         tm = idx.mean_timing()
@@ -814,6 +843,7 @@ def main():
         ms_step = ms_total / steps
         res = {"B": B, "ms_per_step": ms_step, "qps": B / (ms_step * 1e-3), "scan_us": scan_us_max, "calls": tm["calls"],
                "launches": int(launches), "launches_per_step": tm["launches"], "clocks": clocks, "steps": steps, "out": o,
+               "last": last,
                "kernel": "scan_tc_kernel" if B > 4 else "scan_stream_kernel"}
         if with_e2e:
             q_host = q_dev.cpu().pin_memory()
@@ -967,6 +997,8 @@ def main():
                 except Exception as e:
                     enc["cpu_baseline"] = {"error": repr(e)[:200]}
             line["encoder"] = enc
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, *head["last"])
         emit(line)
     if world > 1:
         dist.barrier()
@@ -974,6 +1006,7 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True     # the checkout may be read-only: the bench writes nothing into it
     try:
         main()
     except BaseException as exc:      # a rank that dies must take the job down (torchrun then stops the others): never hang

@@ -45,3 +45,27 @@ def test_clock_sampler_parses_nvidia_smi_lines():
                (102.0, "0, 1965, 1965, 150.0, 0x0, Not Active, Not Active, Not Active, Not Active")]    # after it
     c = s.stop()
     assert c["samples"] == 3 and c["sm_mhz"] == 1470.0 and c["sm_max_mhz"] == 1965.0 and c["reasons"] == ["sw_power_cap"]
+
+
+def test_dump_outputs_writes_float_arrays_and_samples_large_outputs(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    g = torch.Generator().manual_seed(0)
+    raw = torch.rand((1024, 10), generator=g).sort(dim=1, descending=True).values
+    ids = torch.randint(0, 100_000_000, (1024, 10), generator=g)
+    bench.dump_outputs(str(tmp_path / "all"), raw * 1.5, raw, ids)
+    got = {f.stem: np.load(f) for f in (tmp_path / "all").iterdir()}
+    assert sorted(got) == ["ids", "raw_scores", "scores"]
+    assert got["ids"].dtype == np.float64 and np.array_equal(got["ids"], ids.numpy())
+    assert got["scores"].dtype == got["raw_scores"].dtype == np.float32 and np.array_equal(got["raw_scores"], raw.numpy())
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 16 << 10)
+    for name in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / name), raw * 1.5, raw, ids)
+    s1 = {f.stem: np.load(f) for f in (tmp_path / "s1").iterdir()}
+    s2 = {f.stem: np.load(f) for f in (tmp_path / "s2").iterdir()}
+    rows = s1["query_rows"].astype(np.int64)
+    assert sum(a.nbytes for a in s1.values()) <= 16 << 10 and len(rows) > 0 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(s1["ids"], ids.numpy()[rows]) and np.array_equal(s1["scores"], (raw * 1.5).numpy()[rows])
+    assert all(np.array_equal(s1[k], s2[k]) for k in s1)      # the sample is fixed

@@ -37,14 +37,23 @@ def _check_line(d, n_gpus):
     assert isinstance(d["env"], dict)
 
 
-def test_bench_line_contract_and_checks_one_gpu():
+def test_bench_line_contract_and_checks_one_gpu(tmp_path):
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
     cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--rows", "4000000", "--steps", "3", "--warmup", "3",
-           "--no-encoder", "--no-cpu-baseline"]
+           "--no-encoder", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=900, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-3000:]
     lines = [l for l in out.stdout.splitlines() if l.strip()]
     assert len(lines) == 1, out.stdout[-2000:]
     _check_line(json.loads(lines[0]), 1)
+    # the dumped results are the checked ones: planted rows first, scores sorted
+    d = {n: np.load(tmp_path / f"{n}.npy") for n in ("scores", "raw_scores", "ids")}
+    assert all(a.shape == (1024, 10) for a in d.values()) and d["ids"].dtype == np.float64
+    pos, gids = bench.planted_ids(1024, 4_000_000)
+    assert np.array_equal(d["ids"][pos, 0], np.asarray(gids, np.float64))
+    assert np.all(np.diff(d["scores"], axis=1) <= 0)
 
 
 def test_bench_line_contract_and_checks_multi_gpu():

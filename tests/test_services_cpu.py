@@ -67,7 +67,7 @@ def test_build_tool_records_match_reference():
         assert b._calculate_optimal_batch_size(int(n)) == want
 
 
-def test_embedding_service_text_rules_and_errors():
+def test_embedding_service_text_rules_and_errors(monkeypatch):
     E = importlib.import_module("rag-project-icd10_b200.services.embedding_service")
     g = _golden("embedding_service_golden.json")
 
@@ -90,8 +90,8 @@ def test_embedding_service_text_rules_and_errors():
 
     old = E.EmbeddingService.engine_factory
     E.EmbeddingService.engine_factory = Rec
-    os.environ["EMBEDDING_MODEL_NAME"] = "shibing624/text2vec-base-chinese"
-    os.environ["EMBEDDING_DEVICE"] = "cpu"
+    monkeypatch.setenv("EMBEDDING_MODEL_NAME", "shibing624/text2vec-base-chinese")
+    monkeypatch.setenv("EMBEDDING_DEVICE", "cpu")       # restored afterwards: later GPU tests build services on cuda
     try:
         es = E.EmbeddingService()
         probe = ["急性胃肠炎", "query: 已带前缀", "passage: 已带前缀", "", " 前导空格", "Query: 大写不算"]

@@ -201,11 +201,12 @@ def _build_worker(rank, world, port, work, q):
     dist.destroy_process_group()
 
 
-def test_sharded_build_writes_the_same_files_as_a_single_process_build(tmp_path):
+def test_sharded_build_writes_the_same_files_as_a_single_process_build(tmp_path, monkeypatch):
     """tools/build_database.py with the records split over 2 ranks (gloo, fake encoder / device table): rank 0 writes the
     scalar columns and commits, every rank fills its slice of the vector files; the result is byte-identical to the
     single-process build and every rank ends up serving rows shard_bounds(n, r, 2)."""
     import torch.multiprocessing as mp
+    monkeypatch.chdir(tmp_path)     # the builder appends to ./logs/database_build.log; the workers inherit the directory
     os.environ["PYTHONHASHSEED"] = "0"
     src = open(os.path.join(ROOT, "data", "ICD_10v601.csv"), encoding="utf-8-sig").read().splitlines()
     (tmp_path / "subset.csv").write_text("﻿" + "\n".join(src[:702]) + "\n", encoding="utf-8")
