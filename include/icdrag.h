@@ -123,6 +123,15 @@ int icd_index_read(const icd_index* idx, int64_t row0, int64_t n, float* out);
 int icd_index_search(icd_index* idx, const void* q, int q_dtype, int B, int k, int weight_mode,
                      int path, float* out_score, float* out_raw, int64_t* out_id, void* stream,
                      int sync);
+/* filtered search: the exact top-k over the rows a bitmap allows (a scalar `filter` expression evaluated on the host).
+ *   row_mask   ceil(n/32) uint32 words, host or device (bit i&31 of word i>>5 = local row i may be returned); bits at or
+ *              above n are ignored; NULL = all rows (== icd_index_search)
+ *   mask_rows  must equal icd_index_size(idx), else ICD_E_ARG
+ * Ordering, weight modes and the (-inf, -1) tail (fewer than k allowed rows) as icd_index_search.  A host mask is
+ * copied into the handle's workspace like the queries. */
+int icd_index_search_filtered(icd_index* idx, const void* q, int q_dtype, int B, int k, int weight_mode, int path,
+                              const uint32_t* row_mask, int64_t mask_rows, float* out_score, float* out_raw,
+                              int64_t* out_id, void* stream, int sync);
 /* kernels launched / microseconds of device time of the last search on this handle, split by
  * stage: [0] scan, [1] merge, [2] rescore+finalise.  For bench.py's roofline line. */
 int icd_index_last_timing(const icd_index* idx, float* us3, int* launches);
@@ -148,6 +157,11 @@ int icd_shard_group_import_slabs(icd_shard_group* g, const void* handles /*[worl
 int icd_shard_group_search(icd_shard_group* g, const void* q, int q_dtype, int B, int k,
                            int weight_mode, int path, int exchange, float* out_score,
                            float* out_raw, int64_t* out_id, void* stream, int sync);
+/* the same with a row mask over this rank's LOCAL rows (mask_rows == icd_index_size of the local table); every rank
+ * passes the mask of its own rows, results carry global ids as above */
+int icd_shard_group_search_filtered(icd_shard_group* g, const void* q, int q_dtype, int B, int k, int weight_mode,
+                                    int path, int exchange, const uint32_t* row_mask, int64_t mask_rows,
+                                    float* out_score, float* out_raw, int64_t* out_id, void* stream, int sync);
 
 /* ---------------------------------------------------------------- encoder ------------------
  * Replaces the arithmetic of SentenceTransformer.encode(normalize_embeddings=True)

@@ -28,9 +28,10 @@ SYMBOLS = [
     "icd_version", "icd_last_error", "icd_launch_count", "icd_device_count", "icd_tune",
     "icd_index_create", "icd_index_destroy", "icd_index_append", "icd_index_adopt", "icd_index_clear",
     "icd_index_size", "icd_index_dim", "icd_index_read", "icd_index_search", "icd_index_last_timing",
-    "icd_index_set_timing", "icd_index_mean_timing",
+    "icd_index_set_timing", "icd_index_mean_timing", "icd_index_search_filtered",
     "icd_nccl_unique_id", "icd_shard_group_create", "icd_shard_group_destroy",
     "icd_shard_group_export_slab", "icd_shard_group_import_slabs", "icd_shard_group_search",
+    "icd_shard_group_search_filtered",
     "icd_encoder_weight_count", "icd_encoder_create", "icd_encoder_destroy", "icd_encoder_reserve",
     "icd_encoder_forward", "icd_encoder_read_hidden", "icd_encoder_set_token_head", "icd_encoder_token_logits",
     "icd_tokenizer_create", "icd_tokenizer_destroy", "icd_tokenizer_encode", "icd_pack_batch",
@@ -109,6 +110,7 @@ def _declare(L: C.CDLL) -> None:
     L.icd_index_dim.argtypes = [vp]
     L.icd_index_read.argtypes = [vp, i64, i64, vp]
     L.icd_index_search.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, i32]
+    L.icd_index_search_filtered.argtypes = [vp, vp, i32, i32, i32, i32, i32, vp, i64, vp, vp, vp, vp, i32]
     L.icd_index_last_timing.argtypes = [vp, f32p, C.POINTER(i32)]
     L.icd_index_set_timing.argtypes = [vp, i32]
     L.icd_index_mean_timing.argtypes = [vp, f32p, C.POINTER(i32)]
@@ -119,6 +121,7 @@ def _declare(L: C.CDLL) -> None:
         L.icd_shard_group_export_slab.argtypes = [vp, vp]
         L.icd_shard_group_import_slabs.argtypes = [vp, vp]
         L.icd_shard_group_search.argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, vp, vp, i32]
+        L.icd_shard_group_search_filtered.argtypes = [vp, vp, i32, i32, i32, i32, i32, i32, vp, i64, vp, vp, vp, vp, i32]
     if hasattr(L, "icd_encoder_create"):
         L.icd_encoder_weight_count.argtypes = [C.POINTER(BertCfg)]
         L.icd_encoder_weight_count.restype = i64
@@ -187,6 +190,23 @@ def vec_dtype(x) -> int:
     if x.dtype == np.uint16:
         return BF16
     raise TypeError(f"unsupported array dtype {x.dtype}")
+
+
+def mask_ptr(mask, n_rows: int) -> int:
+    """Address of a packed row mask (engine/filter_expr.py::pack_bits): uint32 words, numpy or a CUDA tensor, at least
+    ceil(n_rows / 32) of them.  0 for None (every row)."""
+    if mask is None:
+        return 0
+    words = (int(n_rows) + 31) // 32
+    if _is_torch(mask):
+        import torch
+        if mask.dtype not in (torch.uint32, torch.int32):
+            raise TypeError(f"row mask must be uint32 words, got {mask.dtype}")
+    elif not isinstance(mask, np.ndarray) or mask.dtype not in (np.uint32, np.int32):
+        raise TypeError("row mask must be a uint32 numpy array or tensor (engine/filter_expr.py::pack_bits)")
+    if mask.ndim != 1 or int(mask.shape[0]) < words:
+        raise ValueError(f"row mask of {n_rows} rows needs {words} uint32 words, got shape {tuple(mask.shape)}")
+    return buf_ptr(mask)
 
 
 def current_stream_ptr(device_index: Optional[int] = None) -> int:

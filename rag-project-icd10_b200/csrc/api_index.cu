@@ -86,7 +86,7 @@ static int alloc_table(icd_index* x, int64_t cap) {
 // Writes [B, k] results into the given DEVICE buffers (any may be null).
 int index_search_device(icd_index* x, int B, int k, int weight_mode, int path, int64_t row_offset,
                         float* d_score, float* d_raw, int64_t* d_id, uint8_t* d_level,
-                        bool q_exact_bf16, const PushTargets* push, cudaStream_t st) {
+                        bool q_exact_bf16, const PushTargets* push, const uint32_t* d_mask, cudaStream_t st) {
   const int64_t n = x->n;
   const bool have_master = x->master != nullptr;
   const int weight_pre = weight_mode == ICD_WEIGHT_PRE ? 1 : 0;
@@ -150,6 +150,7 @@ int index_search_device(icd_index* x, int B, int k, int weight_mode, int path, i
       a.part_id = (int*)x->part_id.ptr;
       a.P = P;
       a.groups_used = &P_used;
+      a.mask = d_mask;
       // [B] pruning bounds followed by the zeroed drift-limiter counters (two regions: pre-pass, main)
       const int prog_ints = tensor_scan_progress_ints();
       ICD_TRY(x->gbound.reserve(((size_t)B + 2 * prog_ints) * 4));
@@ -206,6 +207,7 @@ int index_search_device(icd_index* x, int B, int k, int weight_mode, int path, i
         a.part_score = (float*)x->part_score.ptr;
         a.part_id = (int*)x->part_id.ptr;
         a.P = P;
+        a.mask = d_mask;
         ICD_TRY(launch_stream_scan(a, st));
       }
     }
@@ -276,6 +278,24 @@ int index_stage_queries(icd_index* x, const void* q, int q_dtype, int B, cudaStr
     set_error("unknown query dtype %d", q_dtype);
     return ICD_E_ARG;
   }
+  return ICD_OK;
+}
+
+int index_stage_mask(icd_index* x, const uint32_t* row_mask, int64_t mask_rows, const uint32_t** d_mask, cudaStream_t st) {
+  *d_mask = nullptr;
+  if (!row_mask) return ICD_OK;
+  if (mask_rows != x->n) {
+    set_error("row mask covers %lld rows, the table holds %lld", (long long)mask_rows, (long long)x->n);
+    return ICD_E_ARG;
+  }
+  const size_t bytes = (size_t)((x->n + 31) / 32) * 4;
+  if (is_device_ptr(row_mask)) {
+    *d_mask = row_mask;
+    return ICD_OK;
+  }
+  ICD_TRY(x->mask.reserve(std::max<size_t>(bytes, 16)));
+  if (bytes) ICD_CUDA(cudaMemcpyAsync(x->mask.ptr, row_mask, bytes, cudaMemcpyHostToDevice, st));
+  *d_mask = (const uint32_t*)x->mask.ptr;
   return ICD_OK;
 }
 
@@ -366,6 +386,7 @@ int icd_index_destroy(icd_index* x) {
   x->out_stage.release();
   x->in_stage.release();
   x->gbound.release();
+  x->mask.release();
   x->q_f32_alt.release();
   x->q_bf16_alt.release();
   x->out_stage_alt.release();
@@ -500,7 +521,7 @@ namespace icd {
 constexpr int kPipeChunk = 2048;
 
 static int search_host_pipelined(icd_index* x, const void* q, int q_dtype, int B, int k, int weight_mode, int path,
-                                 float* out_score, float* out_raw, int64_t* out_id, cudaStream_t st) {
+                                 const uint32_t* d_mask, float* out_score, float* out_raw, int64_t* out_id, cudaStream_t st) {
   if (!x->copy_stream) {
     ICD_CUDA(cudaStreamCreateWithFlags(&x->copy_stream, cudaStreamNonBlocking));
     for (int i = 0; i < 2; ++i) {
@@ -559,7 +580,8 @@ static int search_host_pipelined(icd_index* x, const void* q, int q_dtype, int B
       float* d_score = (float*)x->out_stage.ptr;
       float* d_raw = d_score + (size_t)nb * k;
       int64_t* d_id = (int64_t*)(d_raw + (size_t)nb * k);
-      ICD_TRY(index_search_device(x, nb, k, weight_mode, path, 0, d_score, d_raw, d_id, nullptr, q_dtype == ICD_BF16, nullptr, st));
+      ICD_TRY(index_search_device(x, nb, k, weight_mode, path, 0, d_score, d_raw, d_id, nullptr, q_dtype == ICD_BF16, nullptr,
+                                  d_mask, st));
       ICD_CUDA(cudaEventRecord(x->ev_done[s], st));
       ICD_TRY(copy_back(prev));   // the previous chunk's results, while this chunk is being searched
       prev.b0 = b0, prev.nb = nb, prev.set = s, prev.d_score = d_score;
@@ -582,6 +604,13 @@ static int search_host_pipelined(icd_index* x, const void* q, int q_dtype, int B
 
 int icd_index_search(icd_index* x, const void* q, int q_dtype, int B, int k, int weight_mode, int path,
                      float* out_score, float* out_raw, int64_t* out_id, void* stream, int sync) {
+  return icd_index_search_filtered(x, q, q_dtype, B, k, weight_mode, path, nullptr, 0, out_score, out_raw, out_id, stream,
+                                   sync);
+}
+
+int icd_index_search_filtered(icd_index* x, const void* q, int q_dtype, int B, int k, int weight_mode, int path,
+                              const uint32_t* row_mask, int64_t mask_rows, float* out_score, float* out_raw,
+                              int64_t* out_id, void* stream, int sync) {
   ICD_CHECK_ARG(x != nullptr, "index is null");
   ICD_CHECK_ARG(B >= 0, "negative batch");
   ICD_CHECK_ARG(k >= 1 && k <= ICD_MAX_K, "k must be in [1, 128]");
@@ -595,8 +624,10 @@ int icd_index_search(icd_index* x, const void* q, int q_dtype, int B, int k, int
                         (out_id && !is_device_ptr(out_id));
   const bool all_host_out = (!out_score || !is_device_ptr(out_score)) && (!out_raw || !is_device_ptr(out_raw)) &&
                             (!out_id || !is_device_ptr(out_id));
+  const uint32_t* d_mask = nullptr;
+  ICD_TRY(index_stage_mask(x, row_mask, mask_rows, &d_mask, st));
   if (B >= 2 * kPipeChunk && !is_device_ptr(q) && all_host_out && x->n > 0)
-    return search_host_pipelined(x, q, q_dtype, B, k, weight_mode, path, out_score, out_raw, out_id, st);
+    return search_host_pipelined(x, q, q_dtype, B, k, weight_mode, path, d_mask, out_score, out_raw, out_id, st);
   constexpr int kMaxBatch = 8192;  // bounds the workspace; larger batches run as several passes
   for (int b0 = 0; b0 < B; b0 += kMaxBatch) {
     const int nb = std::min(kMaxBatch, B - b0);
@@ -614,7 +645,7 @@ int icd_index_search(icd_index* x, const void* q, int q_dtype, int B, int k, int
     float* k_raw = (o_raw && is_device_ptr(o_raw)) ? o_raw : (o_raw ? d_raw : nullptr);
     int64_t* k_id = (o_id && is_device_ptr(o_id)) ? o_id : (o_id ? d_id : nullptr);
     ICD_TRY(index_search_device(x, nb, k, weight_mode, path, 0, k_score, k_raw, k_id, nullptr,
-                                q_dtype == ICD_BF16, nullptr, st));
+                                q_dtype == ICD_BF16, nullptr, d_mask, st));
     ICD_TRY(copy_out(o_score, k_score, (size_t)nb * k * 4, st));
     ICD_TRY(copy_out(o_raw, k_raw, (size_t)nb * k * 4, st));
     ICD_TRY(copy_out(o_id, k_id, (size_t)nb * k * 8, st));

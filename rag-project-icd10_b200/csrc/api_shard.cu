@@ -215,6 +215,13 @@ int icd_shard_group_import_slabs(icd_shard_group* g, const void* handles) {
 
 int icd_shard_group_search(icd_shard_group* g, const void* q, int q_dtype, int B, int k, int weight_mode, int path,
                            int exchange, float* out_score, float* out_raw, int64_t* out_id, void* stream, int sync) {
+  return icd_shard_group_search_filtered(g, q, q_dtype, B, k, weight_mode, path, exchange, nullptr, 0, out_score, out_raw,
+                                         out_id, stream, sync);
+}
+
+int icd_shard_group_search_filtered(icd_shard_group* g, const void* q, int q_dtype, int B, int k, int weight_mode,
+                                    int path, int exchange, const uint32_t* row_mask, int64_t mask_rows,
+                                    float* out_score, float* out_raw, int64_t* out_id, void* stream, int sync) {
   ICD_CHECK_ARG(g != nullptr, "group is null");
   ICD_CHECK_ARG(B >= 0 && B <= kSlabMaxB, "batch must be in [0, 8192] per call");
   ICD_CHECK_ARG(k >= 1 && k <= ICD_MAX_K, "k must be in [1, 128]");
@@ -235,6 +242,8 @@ int icd_shard_group_search(icd_shard_group* g, const void* q, int q_dtype, int B
     return ICD_E_STATE;
   }
   ICD_TRY(index_stage_queries(x, q, q_dtype, B, st));
+  const uint32_t* d_mask = nullptr;   // this rank's local rows
+  ICD_TRY(index_stage_mask(x, row_mask, mask_rows, &d_mask, st));
   const size_t nk = (size_t)B * k;
   const int local_mode = (weight_mode == ICD_WEIGHT_PRE) ? ICD_WEIGHT_PRE : ICD_WEIGHT_NONE;
 
@@ -275,7 +284,7 @@ int icd_shard_group_search(icd_shard_group* g, const void* q, int q_dtype, int B
     int64_t* s_id = W == 1 ? (int64_t*)g->recv_id.ptr : (int64_t*)g->send_id.ptr;
     uint8_t* s_lv = W == 1 ? (uint8_t*)g->recv_lv.ptr : (uint8_t*)g->send_lv.ptr;
     ICD_TRY(index_search_device(x, B, k, local_mode, path, g->row_offset, nullptr, s_raw, s_id, s_lv,
-                                q_dtype == ICD_BF16, nullptr, st));
+                                q_dtype == ICD_BF16, nullptr, d_mask, st));
     if (W > 1) {
       ICD_NCCL(g_nccl.GroupStart());
       ICD_NCCL(g_nccl.AllGather(s_raw, g->recv_raw.ptr, nk * 4, /*ncclInt8*/ 0, g->comm, st));
@@ -303,7 +312,7 @@ int icd_shard_group_search(icd_shard_group* g, const void* q, int q_dtype, int B
     }
     push.epoch = g->epoch;
     ICD_TRY(index_search_device(x, B, k, local_mode, path, g->row_offset, nullptr, nullptr, nullptr, nullptr,
-                                q_dtype == ICD_BF16, &push, st));
+                                q_dtype == ICD_BF16, &push, d_mask, st));
     // consumer: sources are the blocks [parity][0..W) of the local slab; fields are strided by block
     char* base = g->slab + L.block(parity, 0);
     f.cand_score = (const float*)(base + L.blk_raw);

@@ -33,6 +33,7 @@ struct icd_index {
   int map_gen = -1;
   // workspace
   icd::DeviceBuf q_f32, q_bf16, part_score, part_id, cand_score, cand_id, out_stage, in_stage, gbound;
+  icd::DeviceBuf mask;   // a row mask handed over in host memory, copied in like the queries
   // pipelined searches from host buffers (icd_index_search, large batches): the second set of query / result staging
   // buffers, the copy stream and the events that order the two streams
   icd::DeviceBuf q_f32_alt, q_bf16_alt, out_stage_alt;
@@ -52,6 +53,9 @@ namespace icd {
 int index_stage_queries(icd_index* x, const void* q, int q_dtype, int B, cudaStream_t st);
 int index_search_device(icd_index* x, int B, int k, int weight_mode, int path, int64_t row_offset,
                         float* d_score, float* d_raw, int64_t* d_id, uint8_t* d_level,
-                        bool q_exact_bf16, const PushTargets* push, cudaStream_t st);
+                        bool q_exact_bf16, const PushTargets* push, const uint32_t* d_mask, cudaStream_t st);
+// row mask of a filtered search: checks mask_rows == x->n, copies a host mask into the workspace; *d_mask = the device
+// mask, or null when row_mask is null (every row)
+int index_stage_mask(icd_index* x, const uint32_t* row_mask, int64_t mask_rows, const uint32_t** d_mask, cudaStream_t st);
 int copy_out(void* dst, const void* src_dev, size_t bytes, cudaStream_t st);
 }  // namespace icd

@@ -20,6 +20,7 @@ struct StreamScanArgs {
   float* part_score;  // [B, P, k]
   int* part_id;       // [B, P, k] local row, -1 = empty
   int P;              // partial lists per query == grid size
+  const uint32_t* mask;  // row bitmap (bit i & 31 of word i >> 5 = row i may be returned), null = every row
 };
 int stream_scan_grid();
 int stream_scan_max_queries(bool f32rows, int dim);
@@ -44,6 +45,7 @@ struct TensorScanArgs {
   int tile_stride;    // 0/1: scan every row; s > 1: scan every s-th 128-row tile only (sampling pre-pass)
   int pre_slots;      // != 0 (with tile_stride > 1): slot-maxima pre-pass -- part_score receives [B, groups, tensor_scan_pre_slots()]
                       // running maxima instead of sorted lists, part_id is untouched; feed launch_bound_from_slots
+  const uint32_t* mask;  // row bitmap as StreamScanArgs::mask, null = every row
 };
 int tensor_scan_pre_slots();
 int tensor_scan_pre_capacity();   // largest kc the slot-maxima bound serves (slots x the row-group classes it keeps apart)

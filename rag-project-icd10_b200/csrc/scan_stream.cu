@@ -85,12 +85,15 @@ __device__ __forceinline__ float warp_list_insert(float* sc, int* id, int k, flo
   return sc[k - 1];
 }
 
-// NQ queries per pass, CPL 16-byte chunks per lane per row, R rows in flight per warp.
-template <int NQ, int CPL, bool F32ROWS, int R>
+// NQ queries per pass, CPL 16-byte chunks per lane per row, R rows in flight per warp.  MASKED: only rows whose bit is
+// set in `mask` are read and inserted (a template parameter: the widest variants have no register to spare, so the
+// unfiltered scan stays exactly what it was).
+template <int NQ, int CPL, bool F32ROWS, int R, bool MASKED>
 __global__ void __launch_bounds__(kWarps * 32, 2)
 scan_stream_kernel(const void* __restrict__ table, const uint8_t* __restrict__ levels, int64_t n_rows,
                    int dim, const float* __restrict__ q, int nq_valid, int k, int weight_pre,
-                   float* __restrict__ part_score, int* __restrict__ part_id, int q0, int P) {
+                   float* __restrict__ part_score, int* __restrict__ part_id, int q0, int P,
+                   const uint32_t* __restrict__ mask) {
   constexpr int E = RowChunk<F32ROWS>::kElems;
   constexpr int kRowsPerWarpIter = R;
   constexpr int kRowsPerCtaIter = kWarps * R;
@@ -127,10 +130,19 @@ scan_stream_kernel(const void* __restrict__ table, const uint8_t* __restrict__ l
 #pragma unroll
   for (int b = 0; b < NQ; ++b) thr[b] = -INFINITY;
 
+  // Row mask: the R rows of a warp step lie in one mask word (R divides 32 and wrow is a multiple of R).  The word of
+  // the next step is loaded one step ahead, so its L2 round trip does not stand in front of the row loads.
+  auto mask_bits = [&](int64_t wrow) -> uint32_t {
+    if constexpr (!MASKED) return 0xffffffffu;
+    return wrow < n_rows ? __ldg(mask + (wrow >> 5)) >> (wrow & 31) : 0u;
+  };
   const char* base = reinterpret_cast<const char*>(table);
+  uint32_t next_bits = mask_bits((int64_t)blockIdx.x * kRowsPerCtaIter + warp * kRowsPerWarpIter);
   for (int64_t row0 = (int64_t)blockIdx.x * kRowsPerCtaIter; row0 < n_rows;
        row0 += (int64_t)gridDim.x * kRowsPerCtaIter) {
     const int64_t wrow = row0 + warp * kRowsPerWarpIter;
+    const uint32_t bits = next_bits;
+    if constexpr (MASKED) next_bits = mask_bits(wrow + (int64_t)gridDim.x * kRowsPerCtaIter);
     uint4 v[kRowsPerWarpIter][CPL];
 #pragma unroll
     for (int r = 0; r < kRowsPerWarpIter; ++r) {
@@ -138,7 +150,7 @@ scan_stream_kernel(const void* __restrict__ table, const uint8_t* __restrict__ l
 #pragma unroll
       for (int i = 0; i < CPL; ++i) {
         const int c = lane + 32 * i;
-        if (row < n_rows && c < nchunks)
+        if (row < n_rows && c < nchunks && (!MASKED || ((bits >> r) & 1u)))
           v[r][i] = ld_stream_u4(base + (size_t)row * row_bytes + (size_t)c * 16);
         else
           v[r][i] = make_uint4(0, 0, 0, 0);
@@ -148,6 +160,7 @@ scan_stream_kernel(const void* __restrict__ table, const uint8_t* __restrict__ l
     for (int r = 0; r < kRowsPerWarpIter; ++r) {
       const int64_t row = wrow + r;
       if (row >= n_rows) break;  // warp-uniform
+      if (MASKED && !((bits >> r) & 1u)) continue;
       float acc[NQ];
 #pragma unroll
       for (int b = 0; b < NQ; ++b) acc[b] = 0.f;
@@ -207,10 +220,10 @@ scan_stream_kernel(const void* __restrict__ table, const uint8_t* __restrict__ l
 
 template <int NQ, int CPL, bool F32ROWS, int R>
 int launch_one(const StreamScanArgs& a, int grid, size_t smem, cudaStream_t st) {
-  auto kern = scan_stream_kernel<NQ, CPL, F32ROWS, R>;
+  auto kern = a.mask ? scan_stream_kernel<NQ, CPL, F32ROWS, R, true> : scan_stream_kernel<NQ, CPL, F32ROWS, R, false>;
   ICD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<grid, kWarps * 32, smem, st>>>(a.table, a.levels, a.n_rows, a.dim, a.q, a.nq, a.k,
-                                        a.weight_pre, a.part_score, a.part_id, a.q0, a.P);
+                                        a.weight_pre, a.part_score, a.part_id, a.q0, a.P, a.mask);
   count_launch();
   ICD_CUDA(cudaGetLastError());
   return ICD_OK;

@@ -90,6 +90,7 @@ struct ScanParams {
   int tstride;   // scan every tstride-th row tile only (1 = all rows; > 1 = the sampling pre-pass)
   int* progress; // [G * T] tiles issued by each CTA's producer (drift limiter), or null
   int drift;     // a producer may run at most this many tiles ahead of the slowest CTA of its row group
+  const uint32_t* mask;  // row bitmap (bit i & 31 of word i >> 5 = row i may be returned), or null = every row
 #ifdef ICD_PROFILING
   int tiled;     // timing experiment: read the table AS IF it were stored tile-major [tile][K block][128 rows][64]
                  // (8 KiB contiguous runs per K block instead of 768-byte row segments); results are meaningless
@@ -128,6 +129,18 @@ __device__ __noinline__ uint2 drain_queue(float* ls, int* li, int kc, int cnt, f
   return make_uint2(__float_as_uint(thr), (uint32_t)cnt);
 }
 
+// The four mask words of the 128-row tile starting at row0 (a multiple of 128); words past the end of the mask
+// (ceil(n_rows / 32) words) read as 0.  Unmasked instantiations see compile-time all-ones words, so every mask test
+// folds away and they are the unfiltered kernel.
+template <bool MASKED>
+__device__ __forceinline__ uint4 tile_mask(const uint32_t* mask, int64_t row0, int64_t n_rows) {
+  if constexpr (!MASKED) return make_uint4(0xffffffffu, 0xffffffffu, 0xffffffffu, 0xffffffffu);
+  const uint32_t* w = mask + (row0 >> 5);
+  return make_uint4(row0 < n_rows ? __ldg(w) : 0u, row0 + 32 < n_rows ? __ldg(w + 1) : 0u,
+                    row0 + 64 < n_rows ? __ldg(w + 2) : 0u, row0 + 96 < n_rows ? __ldg(w + 3) : 0u);
+}
+__device__ __forceinline__ uint32_t mask_word(const uint4& m, int i) { return i == 0 ? m.x : i == 1 ? m.y : i == 2 ? m.z : m.w; }
+
 // BN = table rows per accumulator tile (MMA N); NC = CTAs per MMA (2 = CTA pair, cta_group::2).
 // KBS / NKBT > 0: the stage shape (K blocks per stage) and the TMEM / shared-memory split of the query tile are
 // compile-time constants for dim = 768, so the MMA issue loop unrolls into ~4 instructions per tcgen05.mma.  The generic
@@ -135,13 +148,15 @@ __device__ __noinline__ uint2 drain_queue(float* ls, int* li, int kc, int cnt, f
 // = ~73 issue cycles per 64-cycle MMA (ncu r02a, B = 256: the elected thread was busy issuing 73 % of the time, waiting
 // for data 3 % and for the epilogue 14 %): the tensor pipe was bounded by instruction issue, not by operands.
 //
+// MASKED = a row mask (p.mask) restricts the rows that may be returned (filtered search).  A template parameter: as a
+// run-time branch it cost the epilogue-bound small table (40 474 rows, B = 1024) 9 % with no mask (r03, filter_ab.py).
 // PRE = the sampling pre-pass.  Its only product is a per-query lower bound of the kc-th best score, so it keeps no
 // candidate lists: the epilogue folds every sampled score into kPreSlots running maxima (slot = accumulator column mod 32;
 // slots partition the sampled rows, so the kc-th largest slot maximum is reached by at least kc distinct rows) with
 // straight-line FMNMX code.  r02h (ncu, 12.5 M rows): the list-based pre-pass spent 0.72 / 0.40 / 0.28 ms at B = 1024 / 256 /
 // 128 -- 5-9 % of the scan it precedes -- almost entirely in the divergent sorted-list inserts of its warm-up (each insert
 // call ~450 cycles for the whole warp, ~2 700 calls per warp); the sampled rows themselves stream in ~0.03 ms.
-template <int BN, int NC, int KBS, int NKBT, bool PRE>
+template <int BN, int NC, int KBS, int NKBT, bool PRE, bool MASKED>
 __global__ void __launch_bounds__(kThreads, 1)
 scan_tc_kernel(const __grid_constant__ CUtensorMap tmap, const ScanParams p) {
   constexpr int kBoxBytes = (BN / NC) * BK * 2;  // this CTA's share of one BN x 64 bf16 tile
@@ -417,8 +432,14 @@ scan_tc_kernel(const __grid_constant__ CUtensorMap tmap, const ScanParams p) {
     float smax[kPreSlots];
 #pragma unroll
     for (int j = 0; j < kPreSlots; ++j) smax[j] = -INFINITY;
+    // masked-out rows contribute -inf: the slots then partition the ALLOWED sampled rows, so the kc-th largest slot
+    // maximum is still reached by >= kc rows that may be returned (the bound stays a lower bound of the filtered
+    // kc-th best); mask words are read one tile ahead like the pruning bound of the main epilogue
+    uint4 next_mw = t0 < t1 ? tile_mask<MASKED>(p.mask, t0 * p.tstride * BN, p.n_rows) : make_uint4(0u, 0u, 0u, 0u);
     int it = 0;
     for (int64_t t = t0; t < t1; ++t, ++it) {
+      const uint4 mw = next_mw;
+      if (t + 1 < t1) next_mw = tile_mask<MASKED>(p.mask, (t + 1) * p.tstride * BN, p.n_rows);
       const int buf = (p.nacc == 2) ? (it & 1) : 0;
       const uint32_t use = (p.nacc == 2) ? (uint32_t)(it >> 1) : (uint32_t)it;
       ptx::mbar_wait(ptx::smem_u32(&tfull_bar[buf]), use & 1);
@@ -440,7 +461,8 @@ scan_tc_kernel(const __grid_constant__ CUtensorMap tmap, const ScanParams p) {
             else ptx::mbar_arrive_cluster(ptx::mapa(ptx::smem_u32(&tempty_bar[buf]), 0));
           }
         }
-        if (valid == BN && !p.weight_pre) {
+        const uint32_t bits = mask_word(mw, c32);
+        if (valid == BN && !p.weight_pre && (!MASKED || bits == 0xffffffffu)) {
 #pragma unroll
           for (int c = 0; c < 32; ++c) smax[c] = fmaxf(smax[c], __uint_as_float(r[c]));
         } else {
@@ -449,7 +471,9 @@ scan_tc_kernel(const __grid_constant__ CUtensorMap tmap, const ScanParams p) {
             const int cc = c32 * 32 + c;
             float sv = __uint_as_float(r[c]);
             if (p.weight_pre) sv *= level_weight_f((cc < valid) ? p.levels[row0 + cc] : (uint8_t)2);
-            smax[c] = fmaxf(smax[c], (cc < valid) ? sv : -INFINITY);  // rows past the end: TMA zero fill
+            // rows past the end (TMA zero fill) and masked-out rows
+            const bool keep = MASKED ? (cc < valid && ((bits >> c) & 1u)) : cc < valid;
+            smax[c] = fmaxf(smax[c], keep ? sv : -INFINITY);
           }
         }
       }
@@ -492,7 +516,12 @@ scan_tc_kernel(const __grid_constant__ CUtensorMap tmap, const ScanParams p) {
     // standing in front of this one's (a bound that is one tile old is still a bound)
     int key = (int)0x80808080;
     if (gb) asm volatile("ld.relaxed.gpu.global.s32 %0, [%1];" : "=r"(key) : "l"(gb));
+    // the row mask likewise: the four words of a tile are loaded while the previous tile is processed.  A masked-out
+    // column fails the admission test below, so it never enters a list and never raises the published bound.
+    uint4 next_mw = t0 < t1 ? tile_mask<MASKED>(p.mask, t0 * p.tstride * BN, p.n_rows) : make_uint4(0u, 0u, 0u, 0u);
     for (int64_t t = t0; t < t1; ++t, ++it) {
+      const uint4 mw = next_mw;
+      if (t + 1 < t1) next_mw = tile_mask<MASKED>(p.mask, (t + 1) * p.tstride * BN, p.n_rows);
       if (gb) {
         // bound proven by any row group: rows strictly below it cannot reach the global top-k
         // (equal scores are still admitted: the id tie-break is decided at the merge)
@@ -539,6 +568,7 @@ scan_tc_kernel(const __grid_constant__ CUtensorMap tmap, const ScanParams p) {
                         fmaxf(__uint_as_float(r[c0 + 2]), __uint_as_float(r[c0 + 3])));
         }
         const float m = fmaxf(fmaxf(fmaxf(m8[0], m8[1]), fmaxf(m8[2], m8[3])), fmaxf(fmaxf(m8[4], m8[5]), fmaxf(m8[6], m8[7])));
+        const uint32_t bits = mask_word(mw, c32);
         if (m > adm) {
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
@@ -548,7 +578,7 @@ scan_tc_kernel(const __grid_constant__ CUtensorMap tmap, const ScanParams p) {
               for (int e = 0; e < 4; ++e) {
                 const int cc = c32 * 32 + 4 * j + e;
                 const float sv = __uint_as_float(r[cc]);
-                if (sv > adm && cc < valid) {
+                if (sv > adm && cc < valid && ((bits >> (4 * j + e)) & 1u)) {
                   qs[qn] = sv;
                   qi[qn] = (int)(row0 + cc);
                   ++qn;
@@ -786,7 +816,7 @@ template <int BN>
 static int resident_pairs(size_t smem) {
   static int cached = 0;
   if (cached) return cached;
-  cudaFuncSetAttribute(scan_tc_kernel<BN, 2, 0, 0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit);
+  cudaFuncSetAttribute(scan_tc_kernel<BN, 2, 0, 0, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit);
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(kSMs);
   cfg.blockDim = dim3(kThreads);
@@ -799,7 +829,7 @@ static int resident_pairs(size_t smem) {
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   int n = 0;
-  if (cudaOccupancyMaxActiveClusters(&n, scan_tc_kernel<BN, 2, 0, 0, false>, &cfg) != cudaSuccess) {
+  if (cudaOccupancyMaxActiveClusters(&n, scan_tc_kernel<BN, 2, 0, 0, false, false>, &cfg) != cudaSuccess) {
     cudaGetLastError();
     n = 0;
   }
@@ -807,9 +837,9 @@ static int resident_pairs(size_t smem) {
   return cached;
 }
 
-template <int BN, int NC, int KBS, int NKBT, bool PRE>
+template <int BN, int NC, int KBS, int NKBT, bool PRE, bool MASKED>
 static int launch_one_pre(const CUtensorMap& tmap, const ScanParams& p, int grid, size_t smem, cudaStream_t st) {
-  auto kernel = scan_tc_kernel<BN, NC, KBS, NKBT, PRE>;
+  auto kernel = scan_tc_kernel<BN, NC, KBS, NKBT, PRE, MASKED>;
   static bool attr_set = false;
   if (!attr_set) {
     ICD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
@@ -836,8 +866,11 @@ static int launch_one_pre(const CUtensorMap& tmap, const ScanParams& p, int grid
 
 template <int BN, int NC, int KBS, int NKBT>
 static int launch_one(const CUtensorMap& tmap, const ScanParams& p, int grid, size_t smem, cudaStream_t st, bool pre) {
-  return pre ? launch_one_pre<BN, NC, KBS, NKBT, true>(tmap, p, grid, smem, st)
-             : launch_one_pre<BN, NC, KBS, NKBT, false>(tmap, p, grid, smem, st);
+  if (p.mask)
+    return pre ? launch_one_pre<BN, NC, KBS, NKBT, true, true>(tmap, p, grid, smem, st)
+               : launch_one_pre<BN, NC, KBS, NKBT, false, true>(tmap, p, grid, smem, st);
+  return pre ? launch_one_pre<BN, NC, KBS, NKBT, true, false>(tmap, p, grid, smem, st)
+             : launch_one_pre<BN, NC, KBS, NKBT, false, false>(tmap, p, grid, smem, st);
 }
 
 template <int BN>
@@ -942,6 +975,7 @@ static int launch_tensor_scan_bn(const TensorScanArgs& a, const void* map128, cu
     p.nacc = (kTmemCols - p.acc_col0) / BN >= 2 ? 2 : 1;
     p.tstride = tstride;
     p.drift = scan_drift();
+    p.mask = a.mask;
     p.progress = (a.progress && p.drift > 0 && p.T > 1 && launch < 64 && !l2_table) ? a.progress + (size_t)launch * kSMs : nullptr;
 #ifdef ICD_PROFILING
     p.tiled = (tun().tiled && BN == 128) ? 1 : 0;

@@ -77,11 +77,13 @@ class VectorIndex:
 
     # ---------------------------------------------------------------- search
     def search(self, q, k: int, weight_mode: int = N.WEIGHT_RERANK, path: int = N.PATH_AUTO,
-               out: Optional[Tuple] = None, stream: int = 0, sync: bool = True):
+               out: Optional[Tuple] = None, stream: int = 0, sync: bool = True, mask=None):
         """q: [B, dim] float32/bfloat16, numpy (host) or torch (host/device).
 
         Returns (score [B,k] f32, raw [B,k] f32, ids [B,k] i64) in the memory space of q
-        (numpy for numpy, torch tensors on q's device for torch), or fills `out`."""
+        (numpy for numpy, torch tensors on q's device for torch), or fills `out`.
+        mask: packed uint32 row bitmap (engine/filter_expr.py::pack_bits; numpy or a CUDA tensor): the exact top-k over
+        the rows whose bit is set; fewer than k such rows leave a (-inf, -1) tail.  None = every row."""
         if q.ndim == 1:
             q = q[None, :]
         B = int(q.shape[0])
@@ -100,9 +102,11 @@ class VectorIndex:
         else:
             score, raw, ids = out
         with self._lock:
-            N.check(N.lib().icd_index_search(self._h, N.buf_ptr(q), N.vec_dtype(q), B, int(k), int(weight_mode),
-                                             int(path), N.buf_ptr(score), N.buf_ptr(raw), N.buf_ptr(ids),
-                                             C.c_void_p(stream), 1 if sync else 0), "icd_index_search")
+            n = len(self)
+            N.check(N.lib().icd_index_search_filtered(self._h, N.buf_ptr(q), N.vec_dtype(q), B, int(k), int(weight_mode),
+                                                      int(path), N.mask_ptr(mask, n), n, N.buf_ptr(score),
+                                                      N.buf_ptr(raw), N.buf_ptr(ids), C.c_void_p(stream),
+                                                      1 if sync else 0), "icd_index_search")
         return score, raw, ids
 
     def set_timing(self, on: bool) -> None:

@@ -39,7 +39,8 @@ class ShardGroup:
             dist.barrier()
 
     def search(self, q, k: int, weight_mode: int = N.WEIGHT_RERANK, path: int = N.PATH_AUTO, exchange: int = 1,
-               out=None, stream: int = 0, sync: bool = True):
+               out=None, stream: int = 0, sync: bool = True, mask=None):
+        """mask: packed uint32 bitmap of THIS rank's local rows (VectorIndex.search), None = every row."""
         if q.ndim == 1:
             q = q[None, :]
         B = int(q.shape[0])
@@ -55,9 +56,11 @@ class ShardGroup:
                 out = (np.empty((B, k), np.float32), np.empty((B, k), np.float32), np.empty((B, k), np.int64))
         score, raw, ids = out
         with self.index._lock:       # the group searches through the local index's workspace
-            N.check(N.lib().icd_shard_group_search(self._h, N.buf_ptr(q), N.vec_dtype(q), B, int(k), int(weight_mode),
-                                                   int(path), int(exchange), N.buf_ptr(score), N.buf_ptr(raw),
-                                                   N.buf_ptr(ids), C.c_void_p(stream), 1 if sync else 0),
+            n = len(self.index)
+            N.check(N.lib().icd_shard_group_search_filtered(self._h, N.buf_ptr(q), N.vec_dtype(q), B, int(k),
+                                                            int(weight_mode), int(path), int(exchange),
+                                                            N.mask_ptr(mask, n), n, N.buf_ptr(score), N.buf_ptr(raw),
+                                                            N.buf_ptr(ids), C.c_void_p(stream), 1 if sync else 0),
                     "icd_shard_group_search")
         return score, raw, ids
 

@@ -4,7 +4,7 @@
 It offers the slice of the MilvusClient surface the reference touches (has_collection,
 create_schema / add_field, prepare_index_params / add_index, create_collection,
 get_load_state, load_collection, release_collection, drop_collection, get_collection_stats,
-insert, search, close) over:
+insert, search (with a boolean ``filter`` over the scalar fields: engine/filter_expr.py), query, get, close) over:
   * a device-resident vector table searched by libicdrag.so (engine/index.py): bf16 scan copy
     plus an fp32 master, so single-query search is exact fp32 inner product like Milvus FLAT/IP;
   * a COLUMNAR on-disk form next to MILVUS_DB_PATH (format 2), one directory per collection:
@@ -29,11 +29,13 @@ import json
 import mmap
 import os
 import shutil
+from collections import OrderedDict
 from typing import Any, Dict, Iterable, List, Optional, Sequence, Tuple
 
 import numpy as np
 
 from .. import _native as N
+from . import filter_expr
 from .index import VectorIndex
 
 SCALAR_FIELDS = ["code", "preferred_zh", "has_complication", "main_code", "secondary_code", "level",
@@ -419,6 +421,8 @@ class IcdStoreClient:
         self.root = uri + ".icdb" if not uri.endswith(".icdb") else uri
         self.persist = not uri.startswith(("http://", "https://"))
         self.cols: Dict[str, _Collection] = {}
+        # device row masks of recent filter expressions: (collection, expression) -> (committed rows, mask words)
+        self._masks: "OrderedDict[Tuple[str, str], Tuple[int, Any]]" = OrderedDict()
         if self.persist:
             os.makedirs(self.root, exist_ok=True)
             for fn in sorted(os.listdir(self.root)):
@@ -487,6 +491,7 @@ class IcdStoreClient:
         self._write_header(col, 0, [f["field_name"] for f in (schema.fields if schema else [])])
 
     def drop_collection(self, collection_name: str) -> None:
+        self._forget_masks(collection_name)
         col = self.cols.pop(collection_name, None)
         if col is not None:
             if col.index is not None:
@@ -520,6 +525,7 @@ class IcdStoreClient:
         col.loaded = True
 
     def release_collection(self, collection_name: str) -> None:
+        self._forget_masks(collection_name)
         col = self.cols[collection_name]
         if col.index is not None and self.persist:
             col.index.close()          # frees the HBM table; load_collection maps it back from the column files
@@ -568,6 +574,7 @@ class IcdStoreClient:
             raise
         col.rows.commit()
         col.row_hi = len(col.rows)
+        self._forget_masks(col.name)
         return first
 
     def insert(self, collection_name: str, data: Iterable[Dict[str, Any]]) -> Dict[str, Any]:
@@ -636,6 +643,7 @@ class IcdStoreClient:
     def sharded_append_commit(self, collection_name: str, total_rows: int, is_writer: bool) -> None:
         """Phase 3: rank 0 (is_writer) replaces the header; every rank calls this AFTER the writer has (barrier in
         between) to map the committed columns."""
+        self._forget_masks(collection_name)
         col = self.cols[collection_name]
         if is_writer:
             self._write_header(col, int(total_rows))
@@ -649,8 +657,38 @@ class IcdStoreClient:
         shards with GLOBAL row ids; every rank must issue the same searches."""
         self.cols[collection_name].group = group
 
+    # ---------------------------------------------------------------- filters
+    _MASK_CACHE = 8   # masks kept on the device (12.5 MB each at 100 M rows)
+
+    def _forget_masks(self, collection_name: str) -> None:
+        for key in [k for k in self._masks if k[0] == collection_name]:
+            del self._masks[key]
+
+    def _row_mask(self, col: _Collection, expr: str):
+        """Device bitmap of the rows this client serves ([row_lo, row_hi): a shard's LOCAL rows) that satisfy `expr`, or
+        None for an empty expression.  Cached per (collection, expression) while the committed row count holds."""
+        pred = filter_expr.compile(expr)        # ValueError on a bad expression, before any cache lookup
+        if pred.is_all:
+            return None
+        key = (col.name, str(expr).strip())
+        stamp = (len(col.rows), col.row_lo, col.row_hi)
+        hit = self._masks.get(key)
+        if hit is not None and hit[0] == stamp:
+            self._masks.move_to_end(key)
+            return hit[1]
+        import torch
+        words = filter_expr.pack_bits(pred.mask(col.rows, col.row_lo, col.row_hi))
+        dev = torch.from_numpy(words.view(np.int32)).to(torch.device("cuda", self.device))
+        self._masks[key] = (stamp, dev)
+        self._masks.move_to_end(key)
+        while len(self._masks) > self._MASK_CACHE:
+            self._masks.popitem(last=False)
+        return dev
+
     def search(self, collection_name: str, data, limit: int = 10, output_fields: Optional[List[str]] = None,
-               **_kw) -> List[List[Hit]]:
+               filter: str = "", **_kw) -> List[List[Hit]]:
+        """MilvusClient.search; `filter` = a boolean expression over the scalar fields (engine/filter_expr.py): the exact
+        top-`limit` over the rows it allows (fewer hits when fewer rows match).  ValueError on a bad expression."""
         col = self.cols[collection_name]
         if not col.loaded or col.index is None:
             raise N.NativeError(f"collection {collection_name} is not loaded")
@@ -658,12 +696,13 @@ class IcdStoreClient:
         if q.ndim == 1:
             q = q[None, :]
         k = max(1, min(int(limit), N.MAX_K))
+        mask = self._row_mask(col, filter)
         group = getattr(col, "group", None)
         if group is not None:
-            _, raw, ids = group.search(q, k, weight_mode=N.WEIGHT_NONE)
+            _, raw, ids = group.search(q, k, weight_mode=N.WEIGHT_NONE, mask=mask)
             base = 0
         else:
-            _, raw, ids = col.index.search(q, k, weight_mode=N.WEIGHT_NONE)
+            _, raw, ids = col.index.search(q, k, weight_mode=N.WEIGHT_NONE, mask=mask)
             base = col.row_lo
         fields = output_fields or []
         out = []
@@ -678,23 +717,64 @@ class IcdStoreClient:
             out.append(hits)
         return out
 
-    def search_ranked(self, collection_name: str, queries, limit: int):
+    def search_ranked(self, collection_name: str, queries, limit: int, filter: str = ""):
         """Batched search with the level re-rank done on the GPU (ICD_WEIGHT_RERANK: raw top-k, score x w(level),
         stable re-sort -- milvus_service.py:290-314): returns (score [B,k] f32, raw [B,k] f32, ids [B,k] i64 GLOBAL
-        row ids, -1 = no hit) as numpy arrays; scalar fields are fetched lazily through row() / field()."""
+        row ids, -1 = no hit) as numpy arrays; scalar fields are fetched lazily through row() / field().  `filter` as
+        in search()."""
         col = self.cols[collection_name]
         if not col.loaded or col.index is None:
             raise N.NativeError(f"collection {collection_name} is not loaded")
         q = np.ascontiguousarray(np.asarray(queries, dtype=np.float32))
         if q.ndim == 1:
             q = q[None, :]
+        mask = self._row_mask(col, filter)
         group = getattr(col, "group", None)
         if group is not None:
-            return group.search(q, max(1, min(int(limit), N.MAX_K)), weight_mode=N.WEIGHT_RERANK)
-        score, raw, ids = col.index.search(q, max(1, min(int(limit), N.MAX_K)), weight_mode=N.WEIGHT_RERANK)
+            return group.search(q, max(1, min(int(limit), N.MAX_K)), weight_mode=N.WEIGHT_RERANK, mask=mask)
+        score, raw, ids = col.index.search(q, max(1, min(int(limit), N.MAX_K)), weight_mode=N.WEIGHT_RERANK, mask=mask)
         if col.row_lo:
             ids = np.where(ids >= 0, ids + col.row_lo, ids)
         return score, raw, ids
+
+    def _entities(self, col: _Collection, rows, output_fields: Optional[List[str]]) -> List[Dict[str, Any]]:
+        fields = list(output_fields or [])
+        if "*" in fields:
+            fields = [f for f in fields if f != "*"] + [f for f in SCALAR_FIELDS if f not in fields]
+        out = []
+        for g in rows:
+            row = col.rows.cached_row(int(g))
+            ent = {"id": int(g)}
+            for f in fields:
+                if f != "id":
+                    ent[f] = row.get(f)
+            out.append(ent)
+        return out
+
+    def query(self, collection_name: str, filter: str = "", output_fields: Optional[List[str]] = None,
+              ids=None, limit: Optional[int] = None, **_kw) -> List[Dict[str, Any]]:
+        """MilvusClient.query: the rows (ascending id) that satisfy `filter` (and are among `ids` when given), as dicts
+        {"id": row, <field>: value, ...} of output_fields ("*" = every scalar field).  Reads the column files, so a
+        sharded client answers for every row of the collection."""
+        col = self.cols[collection_name]
+        n = len(col.rows)
+        allowed = filter_expr.compile(filter).mask(col.rows, 0, n)
+        if ids is not None:
+            sel = np.zeros(n, bool)
+            want = np.asarray([ids] if np.isscalar(ids) else list(ids), np.int64)
+            sel[want[(want >= 0) & (want < n)]] = True
+            allowed &= sel
+        rows = np.nonzero(allowed)[0]
+        if limit is not None:
+            rows = rows[:max(0, int(limit))]
+        return self._entities(col, rows, output_fields)
+
+    def get(self, collection_name: str, ids, output_fields: Optional[List[str]] = None, **_kw) -> List[Dict[str, Any]]:
+        """MilvusClient.get: the rows with these primary keys (row ids), in the order given; unknown ids are skipped."""
+        col = self.cols[collection_name]
+        n = len(col.rows)
+        want = [ids] if np.isscalar(ids) else list(ids)
+        return self._entities(col, [int(i) for i in want if 0 <= int(i) < n], output_fields)
 
     def row(self, collection_name: str, row_id: int) -> Dict[str, Any]:
         return self.cols[collection_name].rows[row_id]
@@ -703,6 +783,7 @@ class IcdStoreClient:
         return self.cols[collection_name].rows.cached_row(int(row_id)).get(name)
 
     def close(self) -> None:
+        self._masks.clear()
         for col in self.cols.values():
             if col.index is not None:
                 col.index.close()

@@ -17,12 +17,15 @@ class BatchedRetrieval:
         self.milvus_service = milvus_service
         self.hierarchical_similarity = hierarchical_similarity
 
-    def retrieve(self, diagnoses: Sequence[str], top_k: int = 10) -> List[List[Dict[str, Any]]]:
-        """base_search_results of every diagnosis (multi_diagnosis_service.py:152-153, limit top_k * 2)."""
+    def retrieve(self, diagnoses: Sequence[str], top_k: int = 10, filter: str = "") -> List[List[Dict[str, Any]]]:
+        """base_search_results of every diagnosis (multi_diagnosis_service.py:152-153, limit top_k * 2); `filter` restricts
+        every diagnosis's candidates to the rows a scalar expression allows (MilvusService.search_batch)."""
         diagnoses = list(diagnoses)
         if not diagnoses:
             return []
         vectors = self.embedding_service.encode_queries(diagnoses)
+        if filter:
+            return self.milvus_service.search_batch(vectors, top_k * 2, filter=filter)
         return self.milvus_service.search_batch(vectors, top_k * 2)
 
     def retrieve_enhanced(self, diagnoses: Sequence[str], query_entities: Sequence[Dict[str, Any]], top_k: int = 10):

@@ -288,13 +288,15 @@ class MilvusService:
             return False
 
     # reference :271-320
-    def search(self, query_vector: np.ndarray, top_k: int = 10) -> List[Dict[str, Any]]:
+    # extension: `filter` -- a Milvus boolean expression over the scalar fields (e.g. 'code like "J%"', 'level == 3'),
+    # applied inside the scan (exact top_k over the matching rows); an invalid expression is logged and gives []
+    def search(self, query_vector: np.ndarray, top_k: int = 10, filter: str = "") -> List[Dict[str, Any]]:
         try:
             if not self.client.has_collection(collection_name=self.collection_name):
                 logger.error(f"集合 {self.collection_name} 不存在")
                 return []
             results = self.client.search(collection_name=self.collection_name, data=[query_vector.tolist()],
-                                         limit=top_k, output_fields=_OUTPUT_FIELDS)
+                                         limit=top_k, output_fields=_OUTPUT_FIELDS, filter=filter)
             candidates = []
             if results and len(results) > 0:
                 candidates = [self._candidate(hit) for hit in results[0]]
@@ -328,7 +330,7 @@ class MilvusService:
     # extension (SURVEY 8f-1): all diagnoses of a request in ONE scan launch, level re-rank on the GPU
     # (ICD_WEIGHT_RERANK == the sort at :314).  Element b is what search(query_vectors[b], top_k) returns; the hit
     # dicts are built lazily, on access, from the mapped columns -- 10 000 queries do not cost 100 000 dicts up front.
-    def search_batch(self, query_vectors, top_k: int = 10) -> "LazyBatch":
+    def search_batch(self, query_vectors, top_k: int = 10, filter: str = "") -> "LazyBatch":
         try:
             if not self.client.has_collection(collection_name=self.collection_name):
                 logger.error(f"集合 {self.collection_name} 不存在")
@@ -336,7 +338,7 @@ class MilvusService:
             q = np.asarray(query_vectors, dtype=np.float32)
             if q.ndim == 1:
                 q = q[None, :]
-            _score, raw, ids = self.client.search_ranked(self.collection_name, q, top_k)
+            _score, raw, ids = self.client.search_ranked(self.collection_name, q, top_k, filter=filter)
             return LazyBatch(self, raw, ids)
         except Exception as e:
             logger.error(f"搜索失败: {e}")
