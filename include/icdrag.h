@@ -167,12 +167,14 @@ int icd_shard_group_search_filtered(icd_shard_group* g, const void* q, int q_dty
  * Replaces the arithmetic of SentenceTransformer.encode(normalize_embeddings=True)
  * (services/embedding_service.py:81,97-102,120): BERT (post-LN, erf-GELU, learned absolute
  * positions) -> masked mean over tokens -> L2 normalise.  Tokenisation stays on the host.
+ * XLM-RoBERTa encoders (the same layer, positions numbered from pad_token_id + 1) use the same
+ * weight layout plus icd_encoder_set_embedding_ids.
  */
 typedef struct icd_bert_cfg {
   int32_t vocab_size;   /* 21128 for text2vec-base-chinese */
-  int32_t hidden;       /* 768 (must be 768 in this build) */
+  int32_t hidden;       /* 768 or 1024 */
   int32_t layers;       /* 12 */
-  int32_t heads;        /* 12 (head dim must be 64) */
+  int32_t heads;        /* hidden / 64: 12 at 768, 16 at 1024 (head dim must be 64) */
   int32_t intermediate; /* 3072 */
   int32_t max_position; /* 512 */
   int32_t type_vocab;   /* 2 */
@@ -185,6 +187,11 @@ int64_t icd_encoder_weight_count(const icd_bert_cfg* cfg);
 int icd_encoder_create(const float* weights, int64_t count, const icd_bert_cfg* cfg, int device,
                        icd_encoder** out);
 int icd_encoder_destroy(icd_encoder* enc);
+/* Embedding conventions, read at each forward: token t of a sequence reads position row position_offset + t
+ * (0 for BERT; pad_token_id + 1 = 2 for XLM-RoBERTa) and ids outside [0, vocab_size) read row unk_id (3 for
+ * XLM-RoBERTa's <unk>).  Defaults: 0, and unk_id 100 ([UNK] of BERT vocabularies) when vocab_size > 100, else 0;
+ * a negative unk_id restores that default.  S + position_offset must not exceed max_position. */
+int icd_encoder_set_embedding_ids(icd_encoder* enc, int32_t position_offset, int32_t unk_id);
 /* ids [B, S] int32 (0-padded), lens [B] int32 = number of real tokens (attention mask is
  * position < len); out [B, hidden] of out_dtype. S <= 512 (BERT's position table): S <= 128 -- the
  * sentence-transformers max_seq_length of text2vec-base-chinese -- is one tile of the tensor-core

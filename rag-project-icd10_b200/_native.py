@@ -34,6 +34,7 @@ SYMBOLS = [
     "icd_shard_group_search_filtered",
     "icd_encoder_weight_count", "icd_encoder_create", "icd_encoder_destroy", "icd_encoder_reserve",
     "icd_encoder_forward", "icd_encoder_read_hidden", "icd_encoder_set_token_head", "icd_encoder_token_logits",
+    "icd_encoder_set_embedding_ids",
     "icd_tokenizer_create", "icd_tokenizer_destroy", "icd_tokenizer_encode", "icd_pack_batch",
 ]
 MAX_LABELS = 64
@@ -132,6 +133,7 @@ def _declare(L: C.CDLL) -> None:
         L.icd_encoder_read_hidden.argtypes = [vp, i32, vp, i64]
         L.icd_encoder_set_token_head.argtypes = [vp, vp, vp, i32]
         L.icd_encoder_token_logits.argtypes = [vp, vp, vp, i32, i32, vp, vp, i32]
+        L.icd_encoder_set_embedding_ids.argtypes = [vp, i32, i32]
     if hasattr(L, "icd_tokenizer_create"):
         L.icd_tokenizer_create.argtypes = [C.c_char_p, i64, vp, i64, vp, vp, vp, i64, C.POINTER(vp)]
         L.icd_tokenizer_destroy.argtypes = [vp]

@@ -1,8 +1,11 @@
 // api_encoder.cu -- C ABI of the BERT sentence encoder (include/icdrag.h, icd_encoder_*).
 //
 // Stands where SentenceTransformer(...).encode(normalize_embeddings=True) stands in the
-// reference (services/embedding_service.py:61,81,97-102,120).  Weight blob order (fp32, HF
-// BertModel names) -- mirrored by rag-project-icd10_b200/engine/weights.py:
+// reference (services/embedding_service.py:61,81,97-102,120).  Two shapes: hidden 768 / 12 heads (BERT-base) and
+// hidden 1024 / 16 heads (BERT-large, XLM-R-large: the reference's default intfloat/multilingual-e5-large-instruct);
+// XLM-R is the same post-LN encoder with its positions numbered from pad_token_id + 1 and <unk> = 3
+// (icd_encoder_set_embedding_ids).  Weight blob order (fp32, HF BertModel names; XLMRobertaModel has the same ones)
+// -- mirrored by rag-project-icd10_b200/engine/weights.py:
 //   embeddings.word_embeddings.weight        [V, H]
 //   embeddings.position_embeddings.weight    [P, H]
 //   embeddings.token_type_embeddings.weight  [T, H]
@@ -76,6 +79,9 @@ struct icd_encoder {
   // token-classification head (icd_encoder_set_token_head): logits = h W^T + b per token
   float *head_w = nullptr, *head_b = nullptr;
   int head_labels = 0;
+  // icd_encoder_set_embedding_ids: token t of a sequence reads position row pos_offset + t; ids outside the table read unk
+  int pos_offset = 0;
+  int unk = 0;
 };
 
 namespace icd {
@@ -86,6 +92,9 @@ static int64_t weight_count(const icd_bert_cfg& c) {
   n += (int64_t)c.layers * (3 * H * H + 3 * H + H * H + H + 2 * H + I * H + I + H * I + H + 2 * H);
   return n;
 }
+
+// ids outside the embedding table read [UNK] (100 in BERT vocabularies) unless icd_encoder_set_embedding_ids says otherwise
+static int default_unk(const icd_bert_cfg& c) { return c.vocab_size > 100 ? 100 : 0; }
 
 static int dev_alloc(icd_encoder* e, void** p, size_t bytes) {
   ICD_CUDA(cudaMalloc(p, bytes));
@@ -136,7 +145,7 @@ static int reserve_tokens(icd_encoder* e, int max_tokens) {
   ICD_TRY(gemm_make_map_a(e->m_h1, e->h1, M, H));
   ICD_TRY(gemm_make_map_a(e->m_ctx, e->ctx, M, H));
   ICD_TRY(gemm_make_map_a(e->m_f, e->f, M, I));
-  ICD_TRY(attention_make_map(e->m_qkv, e->qkv, M));
+  ICD_TRY(attention_make_map(e->m_qkv, e->qkv, M, H));
   ICD_TRY(gemm_make_map_out(e->m_t, e->t, M, H));
   ICD_TRY(gemm_make_map_out(e->m_qkv_out, e->qkv, M, 3 * H));
   e->max_tokens = M;
@@ -185,7 +194,8 @@ int64_t icd_encoder_weight_count(const icd_bert_cfg* cfg) { return cfg ? weight_
 
 int icd_encoder_create(const float* weights, int64_t count, const icd_bert_cfg* cfg, int device, icd_encoder** out) {
   ICD_CHECK_ARG(weights && cfg && out, "null argument");
-  ICD_CHECK_ARG(cfg->hidden == 768 && cfg->heads == 12, "this build supports hidden=768, heads=12 (head dim 64)");
+  ICD_CHECK_ARG((cfg->hidden == 768 && cfg->heads == 12) || (cfg->hidden == 1024 && cfg->heads == 16),
+                "supported shapes are hidden=768 with heads=12 and hidden=1024 with heads=16 (head dim 64)");
   ICD_CHECK_ARG(cfg->intermediate > 0 && cfg->intermediate % gemm_tile_n() == 0, "intermediate must be a multiple of 256");
   ICD_CHECK_ARG(cfg->layers >= 1 && cfg->vocab_size > 0 && cfg->max_position > 0 && cfg->type_vocab > 0, "bad config");
   ICD_CHECK_ARG(count == weight_count(*cfg), "weight blob size does not match the config");
@@ -202,6 +212,7 @@ int icd_encoder_create(const float* weights, int64_t count, const icd_bert_cfg* 
   icd_encoder* e = new icd_encoder();
   e->cfg = *cfg;
   e->device = device;
+  e->unk = default_unk(*cfg);
   const int64_t H = cfg->hidden, I = cfg->intermediate;
   float* stage = nullptr;
   const int64_t stage_n = std::max<int64_t>(3 * H * H, I * H);
@@ -363,12 +374,12 @@ static int encode_hidden(icd_encoder* e, const int32_t* ids, const int32_t* lens
     ICD_CUDA(cudaMemcpyAsync(e->lens, lens, (size_t)B * 4, cudaMemcpyHostToDevice, st));
     d_lens = e->lens;
   }
-  // ids outside the embedding table read [UNK] (100 in BERT vocabularies) instead of faulting
-  const int unk = e->cfg.vocab_size > 100 ? 100 : 0;
-  ICD_TRY(launch_embed_ln(d_ids, M, S, e->cfg.vocab_size, unk, e->word, e->pos, e->type, e->eg, e->eb, eps, e->h, st));
+  // ids outside the embedding table read the unk row instead of faulting
+  ICD_TRY(launch_embed_ln(d_ids, M, S, e->cfg.vocab_size, e->unk, e->word, e->pos, e->type, e->eg, e->eb, eps, e->h, st,
+                          e->pos_offset, H));
   if (S > 128) {
     size_t stats_bytes = 0;
-    const size_t part_bytes = attention_long_scratch_bytes(B, S, &stats_bytes);
+    const size_t part_bytes = attention_long_scratch_bytes(B, S, &stats_bytes, H);
     if (part_bytes > e->att_part_cap) {
       if (e->att_part) cudaFree(e->att_part);
       e->att_part = nullptr, e->att_part_cap = 0;
@@ -383,12 +394,13 @@ static int encode_hidden(icd_encoder* e, const int32_t* ids, const int32_t* lens
     }
   }
   auto attention = [&]() {
-    return S <= 128 ? launch_attention_tc(e->m_qkv, d_lens, B, S, e->ctx, e->max_tokens, st)
-                    : launch_attention_tc_long(e->m_qkv, d_lens, B, S, e->att_part, e->att_stats, e->ctx, st);
+    return S <= 128 ? launch_attention_tc(e->m_qkv, d_lens, B, S, e->ctx, e->max_tokens, st, H)
+                    : launch_attention_tc_long(e->m_qkv, d_lens, B, S, e->att_part, e->att_stats, e->ctx, st, H);
   };
   const void* final_h = e->h;
-  const bool skinny = e->fused_ln && M <= skinny_max_tokens() && skinny_linear_supported(M, H, H) &&
-                      skinny_linear_supported(M, 3 * H, H) && skinny_linear_supported(M, I, H) && skinny_linear_supported(M, H, I);
+  const bool skinny = e->fused_ln && M <= skinny_max_tokens() && skinny_linear_supported(M, H, H, H) &&
+                      skinny_linear_supported(M, 3 * H, H, H) && skinny_linear_supported(M, I, H, H) &&
+                      skinny_linear_supported(M, H, I, H);
   if (skinny) {
     // A handful of tokens (batch-1 encode_query): the same deferred-LayerNorm dataflow as below, every linear layer
     // as a weight stream over all SMs (skinny_linear.cu); the row statistics are computed by the consumer itself.
@@ -396,18 +408,18 @@ static int encode_hidden(icd_encoder* e, const int32_t* ids, const int32_t* lens
       LayerW* L = e->layers[l];
       const LayerW* P = l ? e->layers[l - 1] : nullptr;
       SkinnyArgs g{};
-      g = SkinnyArgs{e->h, L->wqkv, L->bqkv, P ? L->cqkv : nullptr, nullptr, e->qkv, M, 3 * H, H, EPI_BIAS, P ? 1 : 0, eps};
+      g = SkinnyArgs{e->h, L->wqkv, L->bqkv, P ? L->cqkv : nullptr, nullptr, e->qkv, M, 3 * H, H, EPI_BIAS, P ? 1 : 0, eps, H};
       ICD_TRY(launch_skinny_linear(g, st));
       ICD_TRY(attention());
-      g = SkinnyArgs{e->ctx, L->wo, L->bo_r, P ? P->ln2g : nullptr, e->h, e->t, M, H, H, EPI_BIAS_RESIDUAL, 0, eps};
+      g = SkinnyArgs{e->ctx, L->wo, L->bo_r, P ? P->ln2g : nullptr, e->h, e->t, M, H, H, EPI_BIAS_RESIDUAL, 0, eps, H};
       ICD_TRY(launch_skinny_linear(g, st));
-      g = SkinnyArgs{e->t, L->w1, L->b1, L->c1, nullptr, e->f, M, I, H, EPI_BIAS_GELU, 1, eps};
+      g = SkinnyArgs{e->t, L->w1, L->b1, L->c1, nullptr, e->f, M, I, H, EPI_BIAS_GELU, 1, eps, H};
       ICD_TRY(launch_skinny_linear(g, st));
-      g = SkinnyArgs{e->f, L->w2, L->b2_r, L->ln1g, e->t, e->h, M, H, I, EPI_BIAS_RESIDUAL, 0, eps};
+      g = SkinnyArgs{e->f, L->w2, L->b2_r, L->ln1g, e->t, e->h, M, H, I, EPI_BIAS_RESIDUAL, 0, eps, H};
       ICD_TRY(launch_skinny_linear(g, st));
     }
     LayerW* L = e->layers.back();
-    ICD_TRY(launch_layernorm(e->h, M, L->ln2g, L->ln2b, eps, e->h1, st));
+    ICD_TRY(launch_layernorm(e->h, M, L->ln2g, L->ln2b, eps, e->h1, st, H));
     final_h = e->h1;
   } else if (e->fused_ln) {
     // Deferred LayerNorm: e->h carries the layer input -- normalised for layer 0 (embed_ln), the un-normalised
@@ -439,7 +451,7 @@ static int encode_hidden(icd_encoder* e, const int32_t* ids, const int32_t* lens
       ICD_TRY(launch_gemm_tc(g, st));
     }
     LayerW* L = e->layers.back();
-    ICD_TRY(launch_layernorm(e->h, M, L->ln2g, L->ln2b, eps, e->h1, st));
+    ICD_TRY(launch_layernorm(e->h, M, L->ln2g, L->ln2b, eps, e->h1, st, H));
     final_h = e->h1;
   } else {
     for (size_t l = 0; l < e->layers.size(); ++l) {
@@ -452,14 +464,14 @@ static int encode_hidden(icd_encoder* e, const int32_t* ids, const int32_t* lens
       // t = ctx Wo^T + bo + h ; h1 = LN(t)
       g = GemmArgs{e->m_ctx, L->m_o, L->bo, e->m_h, e->m_t, M, H, H, EPI_BIAS_RESIDUAL};
       ICD_TRY(launch_gemm_tc(g, st));
-      ICD_TRY(launch_layernorm(e->t, M, L->ln1g, L->ln1b, eps, e->h1, st));
+      ICD_TRY(launch_layernorm(e->t, M, L->ln1g, L->ln1b, eps, e->h1, st, H));
       // f = gelu(h1 W1^T + b1)
       g = GemmArgs{e->m_h1, L->m_1, L->b1, nullptr, e->m_f, M, I, H, EPI_BIAS_GELU};
       ICD_TRY(launch_gemm_tc(g, st));
       // t = f W2^T + b2 + h1 ; h = LN(t)
       g = GemmArgs{e->m_f, L->m_2, L->b2, e->m_h1, e->m_t, M, H, I, EPI_BIAS_RESIDUAL};
       ICD_TRY(launch_gemm_tc(g, st));
-      ICD_TRY(launch_layernorm(e->t, M, L->ln2g, L->ln2b, eps, e->h, st));
+      ICD_TRY(launch_layernorm(e->t, M, L->ln2g, L->ln2b, eps, e->h, st, H));
     }
   }
   *final_h_out = final_h;
@@ -476,7 +488,7 @@ int icd_encoder_forward(icd_encoder* e, const int32_t* ids, const int32_t* lens,
                         int out_dtype, void* stream, int sync) {
   ICD_CHECK_ARG(e != nullptr, "encoder is null");
   ICD_CHECK_ARG(B >= 0 && S >= 1 && S <= 512, "need 1 <= S <= 512");
-  ICD_CHECK_ARG(S <= e->cfg.max_position, "S exceeds max_position");
+  ICD_CHECK_ARG(S + e->pos_offset <= e->cfg.max_position, "S + position offset exceeds max_position");
   const int out_flags = out_dtype;
   out_dtype &= 0xff;
   ICD_CHECK_ARG(out_dtype == ICD_F32 || out_dtype == ICD_BF16, "unknown out dtype");
@@ -502,7 +514,7 @@ int icd_encoder_forward(icd_encoder* e, const int32_t* ids, const int32_t* lens,
   const void* final_h = nullptr;
   const int32_t* d_lens = nullptr;
   ICD_TRY(encode_hidden(e, ids, lens, B, S, st, &final_h, &d_lens));
-  ICD_TRY(launch_pool_normalise(final_h, d_lens, B, S, d_out, out_flags, st));
+  ICD_TRY(launch_pool_normalise(final_h, d_lens, B, S, d_out, out_flags, st, H));
   if (host_out) {
     ICD_CUDA(cudaMemcpyAsync(out, d_out, (size_t)B * H * (out_dtype == ICD_F32 ? 4 : 2), cudaMemcpyDeviceToHost, st));
   }
@@ -510,6 +522,15 @@ int icd_encoder_forward(icd_encoder* e, const int32_t* ids, const int32_t* lens,
   // ones are read when the stream gets there -- with sync = 0 the caller keeps them untouched until then (the feeder
   // in engine/encoder.py double-buffers them behind events)
   if (sync || host_out) ICD_CUDA(cudaStreamSynchronize(st));
+  return ICD_OK;
+}
+
+int icd_encoder_set_embedding_ids(icd_encoder* e, int32_t position_offset, int32_t unk_id) {
+  ICD_CHECK_ARG(e != nullptr, "encoder is null");
+  ICD_CHECK_ARG(position_offset >= 0 && position_offset < e->cfg.max_position, "position_offset outside [0, max_position)");
+  ICD_CHECK_ARG(unk_id < e->cfg.vocab_size, "unk_id outside the vocabulary");
+  e->pos_offset = position_offset;
+  e->unk = unk_id < 0 ? default_unk(e->cfg) : unk_id;
   return ICD_OK;
 }
 
@@ -535,7 +556,7 @@ int icd_encoder_token_logits(icd_encoder* e, const int32_t* ids, const int32_t* 
   ICD_CHECK_ARG(e != nullptr, "encoder is null");
   ICD_CHECK_ARG(e->head_labels > 0, "no token head: call icd_encoder_set_token_head first");
   ICD_CHECK_ARG(B >= 0 && S >= 1 && S <= 512, "need 1 <= S <= 512");
-  ICD_CHECK_ARG(S <= e->cfg.max_position, "S exceeds max_position");
+  ICD_CHECK_ARG(S + e->pos_offset <= e->cfg.max_position, "S + position offset exceeds max_position");
   if (B == 0) return ICD_OK;
   ICD_CHECK_ARG(ids && lens && out, "null buffer");
   ICD_CHECK_ARG((int64_t)B * S <= 0x7fffffffLL / 4, "batch too large");
@@ -558,7 +579,7 @@ int icd_encoder_token_logits(icd_encoder* e, const int32_t* ids, const int32_t* 
   const void* final_h = nullptr;
   const int32_t* d_lens = nullptr;
   ICD_TRY(encode_hidden(e, ids, lens, B, S, st, &final_h, &d_lens));
-  ICD_TRY(launch_token_head(final_h, B * S, e->head_w, e->head_b, L, d_out, st));
+  ICD_TRY(launch_token_head(final_h, B * S, e->head_w, e->head_b, L, d_out, st, e->cfg.hidden));
   if (host_out) ICD_CUDA(cudaMemcpyAsync(out, d_out, bytes, cudaMemcpyDeviceToHost, st));
   // host inputs were handed to cudaMemcpyAsync above: pageable buffers are staged before that call returns, pinned
   // ones are read when the stream gets there -- with sync = 0 the caller keeps them untouched until then (the feeder

@@ -28,11 +28,14 @@
 //
 // Sequences of 129 .. 512 tokens (the token-classification path) run the SAME kernel in split-KV mode: a work item is
 // (sequence, head, 128-query tile, 128-key tile); the softmax of an item is local to its key tile, the item stores its
-// normalised partial output as bf16 into a [key tile][padded row][768] buffer plus (row max in the log2 domain, row
+// normalised partial output as bf16 into a [key tile][padded row][H] buffer plus (row max in the log2 domain, row
 // sum) per (key tile, head, row), and attention_combine_kernel merges the <= 4 partials of a row with the weights
 // exp2(m_t - m) sum_t -- the flash-decoding split, so no kernel keeps a running max across tiles.
 //
-// Roofline: HBM (reads the 2304-wide qkv rows once, writes ctx once); the math is ~1 % of a layer.
+// The hidden size H is a template parameter (768: 12 heads, 1024: 16 heads); it sets the qkv row stride 3H, the ctx
+// row stride, the head count and the split-KV buffers.  Tiles, TMEM and shared memory are per head and do not change.
+//
+// Roofline: HBM (reads the 3H-wide qkv rows once, writes ctx once); the math is ~1 % of a layer.
 #include <stdlib.h>
 #include <string.h>
 
@@ -45,9 +48,7 @@
 namespace icd {
 namespace {
 
-constexpr int H = 768;
 constexpr int HD = 64;
-constexpr int kHeads = 12;
 constexpr int kTile = 128;
 constexpr int kSlots = 4;
 constexpr int kTileBytes = kTile * HD * 2;  // 16 KiB
@@ -80,6 +81,7 @@ __device__ __forceinline__ float ex2_approx(float x) {
   return y;
 }
 
+template <int H>
 __global__ void __launch_bounds__(kThreads, 1)
 attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_constant__ CUtensorMap tmap_ctx,
                     const AttParams p) {
@@ -95,6 +97,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
   uint64_t* ofull_bar = bars + 12;       // [4] O ready in TMEM (per O region)
   uint64_t* ofree_bar = bars + 16;       // [4] O region drained by all 128 rows
   uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(bars + 20);
+  constexpr int kHeads = H / HD;
 
   const int n_items = p.tiles * kHeads;
   const int n_local = (n_items - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
@@ -380,13 +383,15 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tmap_qkv, const __grid_c
 }
 
 // merges the <= 4 key-tile partials of every (token, head): out = sum_t w_t O_t / sum_t w_t, w_t = exp2(m_t - max m) sum_t.
-// One thread per (token, head, 8-column chunk); rows are read / written 16 bytes at a time.
-__global__ void __launch_bounds__(96)
+// One thread per (token, head, 8-column chunk) -- H / 8 threads; rows are read / written 16 bytes at a time.
+template <int H>
+__global__ void __launch_bounds__(H / 8)
 attention_combine_kernel(const __nv_bfloat16* __restrict__ part, const float2* __restrict__ stats, int B, int S, int S_pad,
                          int QT, __nv_bfloat16* __restrict__ ctx) {
   ptx::griddep_launch();
   ptx::griddep_wait();
-  const int row = blockIdx.x;            // token row of the [B * S, 768] ctx buffer
+  constexpr int kHeads = H / HD;
+  const int row = blockIdx.x;            // token row of the [B * S, H] ctx buffer
   const int seq = row / S, t = row % S;
   const int head = threadIdx.x >> 3, chunk = threadIdx.x & 7;
   const size_t prow = (size_t)seq * S_pad + t;
@@ -420,16 +425,38 @@ attention_combine_kernel(const __nv_bfloat16* __restrict__ part, const float2* _
 
 }  // namespace
 
-int attention_make_map(void* map128, const void* qkv, int64_t rows) {
-  return make_tmap_bf16_2d(map128, qkv, (uint64_t)rows, (uint64_t)(3 * H), kTile, HD, true);
+static bool supported_hidden(int hidden) {
+  if (hidden == 768 || hidden == 1024) return true;
+  set_error("attention: hidden size %d is not supported (768 or 1024)", hidden);
+  return false;
+}
+
+int attention_make_map(void* map128, const void* qkv, int64_t rows, int hidden) {
+  if (!supported_hidden(hidden)) return ICD_E_ARG;
+  return make_tmap_bf16_2d(map128, qkv, (uint64_t)rows, (uint64_t)(3 * hidden), kTile, HD, true);
+}
+
+template <int H>
+static int launch_packed(const CUtensorMap& tm, const AttParams& p, void* ctx, int64_t ctx_rows, cudaStream_t st) {
+  // ctx store box: the G * S rows a tile owns x one head (64 columns); encoded per launch because it depends on S
+  alignas(128) unsigned char ctx_map[128];
+  ICD_TRY(make_tmap_bf16_2d(ctx_map, ctx, (uint64_t)ctx_rows, (uint64_t)H, (uint32_t)(p.G * p.S), HD, true));
+  CUtensorMap tc;
+  memcpy(&tc, ctx_map, sizeof(tc));
+  ICD_CUDA(cudaFuncSetAttribute(attention_tc_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+  const int grid = std::min(p.tiles * (H / HD), kSMs);
+  ICD_CUDA(launch_chained(attention_tc_kernel<H>, dim3(grid), dim3(kThreads), (size_t)kSmemBytes, st, 1, tm, tc, p));
+  count_launch();
+  return ICD_OK;
 }
 
 int launch_attention_tc(const void* tmap_qkv, const int32_t* lens, int B, int S, void* ctx, int64_t ctx_rows,
-                        cudaStream_t st) {
+                        cudaStream_t st, int hidden) {
   if (S < 1 || S > kTile) {
     set_error("attention: S=%d outside [1, 128]", S);
     return ICD_E_UNSUPPORTED;
   }
+  if (!supported_hidden(hidden)) return ICD_E_ARG;
   AttParams p{};
   p.lens = lens;
   p.B = B;
@@ -444,32 +471,41 @@ int launch_attention_tc(const void* tmap_qkv, const int32_t* lens, int B, int S,
 #endif
   CUtensorMap tm;
   memcpy(&tm, tmap_qkv, sizeof(tm));
-  // ctx store box: the G * S rows a tile owns x one head (64 columns); encoded per launch because it depends on S
-  alignas(128) unsigned char ctx_map[128];
-  ICD_TRY(make_tmap_bf16_2d(ctx_map, ctx, (uint64_t)ctx_rows, (uint64_t)H, (uint32_t)(p.G * S), HD, true));
+  return hidden == 768 ? launch_packed<768>(tm, p, ctx, ctx_rows, st) : launch_packed<1024>(tm, p, ctx, ctx_rows, st);
+}
+
+// split-KV form for 128 < S <= 512: part [QT * B * S_pad, H] bf16 and stats [QT * heads * B * S_pad] float2 are scratch
+size_t attention_long_scratch_bytes(int B, int S, size_t* stats_bytes, int hidden) {
+  const int QT = (S + kTile - 1) / kTile;
+  const size_t rows = (size_t)QT * B * QT * kTile;
+  if (stats_bytes) *stats_bytes = (size_t)QT * (hidden / HD) * B * QT * kTile * sizeof(float2);
+  return rows * hidden * 2;
+}
+
+template <int H>
+static int launch_split(const CUtensorMap& tm, const AttParams& p, void* part, void* ctx, cudaStream_t st) {
+  alignas(128) unsigned char part_map[128];
+  ICD_TRY(make_tmap_bf16_2d(part_map, part, (uint64_t)p.QT * p.B * p.S_pad, (uint64_t)H, (uint32_t)kTile, HD, true));
   CUtensorMap tc;
-  memcpy(&tc, ctx_map, sizeof(tc));
-  ICD_CUDA(cudaFuncSetAttribute(attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  const int grid = std::min(p.tiles * kHeads, kSMs);
-  ICD_CUDA(launch_chained(attention_tc_kernel, dim3(grid), dim3(kThreads), (size_t)kSmemBytes, st, 1, tm, tc, p));
+  memcpy(&tc, part_map, sizeof(tc));
+  ICD_CUDA(cudaFuncSetAttribute(attention_tc_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+  const int grid = std::min(p.tiles * (H / HD), kSMs);
+  ICD_CUDA(launch_chained(attention_tc_kernel<H>, dim3(grid), dim3(kThreads), (size_t)kSmemBytes, st, 1, tm, tc, p));
+  count_launch();
+  ICD_CUDA(launch_chained(attention_combine_kernel<H>, dim3(p.B * p.S), dim3(H / 8), 0, st, 1,
+                          reinterpret_cast<const __nv_bfloat16*>(part), static_cast<const float2*>(p.part_stats), p.B, p.S,
+                          p.S_pad, p.QT, reinterpret_cast<__nv_bfloat16*>(ctx)));
   count_launch();
   return ICD_OK;
 }
 
-// split-KV form for 128 < S <= 512: part [QT * B * S_pad, 768] bf16 and stats [QT * 12 * B * S_pad] float2 are scratch
-size_t attention_long_scratch_bytes(int B, int S, size_t* stats_bytes) {
-  const int QT = (S + kTile - 1) / kTile;
-  const size_t rows = (size_t)QT * B * QT * kTile;
-  if (stats_bytes) *stats_bytes = (size_t)QT * kHeads * B * QT * kTile * sizeof(float2);
-  return rows * H * 2;
-}
-
 int launch_attention_tc_long(const void* tmap_qkv, const int32_t* lens, int B, int S, void* part, void* stats, void* ctx,
-                             cudaStream_t st) {
+                             cudaStream_t st, int hidden) {
   if (S <= kTile || S > 4 * kTile) {
     set_error("attention (split-KV): S=%d outside (128, 512]", S);
     return ICD_E_UNSUPPORTED;
   }
+  if (!supported_hidden(hidden)) return ICD_E_ARG;
   AttParams p{};
   p.lens = lens;
   p.B = B;
@@ -481,18 +517,7 @@ int launch_attention_tc_long(const void* tmap_qkv, const int32_t* lens, int B, i
   p.part_stats = reinterpret_cast<float2*>(stats);
   CUtensorMap tm;
   memcpy(&tm, tmap_qkv, sizeof(tm));
-  alignas(128) unsigned char part_map[128];
-  ICD_TRY(make_tmap_bf16_2d(part_map, part, (uint64_t)p.QT * B * p.S_pad, (uint64_t)H, (uint32_t)kTile, HD, true));
-  CUtensorMap tc;
-  memcpy(&tc, part_map, sizeof(tc));
-  ICD_CUDA(cudaFuncSetAttribute(attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  const int grid = std::min(p.tiles * kHeads, kSMs);
-  ICD_CUDA(launch_chained(attention_tc_kernel, dim3(grid), dim3(kThreads), (size_t)kSmemBytes, st, 1, tm, tc, p));
-  count_launch();
-  ICD_CUDA(launch_chained(attention_combine_kernel, dim3(B * S), dim3(96), 0, st, 1, reinterpret_cast<const __nv_bfloat16*>(part),
-                          reinterpret_cast<const float2*>(stats), B, S, p.S_pad, p.QT, reinterpret_cast<__nv_bfloat16*>(ctx)));
-  count_launch();
-  return ICD_OK;
+  return hidden == 768 ? launch_split<768>(tm, p, part, ctx, st) : launch_split<1024>(tm, p, part, ctx, st);
 }
 
 }  // namespace icd

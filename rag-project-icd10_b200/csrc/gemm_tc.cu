@@ -25,7 +25,8 @@
 // Deferred LayerNorm.  The two LayerNorm launches per layer were 9 % of the encoder (HBM-bound, r01c launch
 // list); they are folded into the GEMMs on either side instead.  A GEMM whose output feeds a LayerNorm
 // (O projection, FFN down) also emits per-row partial (sum, sum of squares) of its 128 output columns per
-// column half -- [N/128][rows] float2, no atomics, deterministic.  A GEMM that READS a LayerNorm output
+// column half -- [N/128][rows] float2, no atomics, deterministic; a consumer adds the SLOTS = H / 128 partials of a row
+// (6 at hidden 768, 8 at 1024: a template parameter, so the sum stays straight-line code).  A GEMM that READS a LayerNorm output
 // takes the un-normalised stream x as A with W' = W diag(gamma) pre-folded on the host and applies
 //   y = rs * (x W'^T) - rs * mu * c + b',   c[n] = sum_k W'[n,k],  b' = b + W beta
 // per row in its epilogue (the identity CUTLASS's gemm+layernorm fusion uses); a residual epilogue that needs
@@ -65,7 +66,6 @@ constexpr int kBoxCols = 64;                    // staging box: 128 rows x 64 bf
 constexpr int kBoxBytes = BM * kBoxCols * 2;    // 16 KiB
 constexpr int kBoxesPerHalf = (BN / 2) / kBoxCols;  // 2
 constexpr int kStagingBoxes = 4;                // 2 column halves x 2 (double-buffered: a store drains while the next box fills)
-constexpr int kStatSlots = 6;                   // LayerNorm row length 768 = 6 column halves of 128
 constexpr int kBiasBytes = 2 * 2 * (BN / 2) * 4;  // [half][bias | second column vector][128] fp32
 template <int NC>
 constexpr int smem_bytes() {
@@ -99,7 +99,8 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
 // loads of the column vectors stalled their first use -- 2 epilogue warps per scheduler cannot hide that).
 //   LNIN: A is an un-normalised stream, apply its row statistics (QKV / FFN-up in deferred-LayerNorm mode)
 //   STATS: emit the row statistics of the output (residual epilogues in deferred-LayerNorm mode)
-template <int NC, int EPI, bool LNIN, bool STATS>
+//   SLOTS: 128-column partials per row of the incoming statistics (hidden size / 128)
+template <int NC, int EPI, bool LNIN, bool STATS, int SLOTS>
 __global__ void __launch_bounds__(kThreads, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                const __grid_constant__ CUtensorMap tmap_out, const __grid_constant__ CUtensorMap tmap_res,
@@ -261,14 +262,14 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
     // the FFN-up GEMM's stall samples): the bias / second-vector element this thread publishes through shared
     // memory and the LayerNorm partials of its row.
     float nx_bias = 0.0f, nx_vec2 = 1.0f;
-    float2 nx_stat[kStatSlots];
+    float2 nx_stat[SLOTS];
     auto request = [&](int t) {
       const int tm0 = (t / n_tiles) * (BM * NC) + (int)rank * BM, tn0 = (t % n_tiles) * BN;
       nx_bias = p.bias[tn0 + half * (BN / 2) + row_in_tile];
       if ((LNIN || with_res) && p.vec2) nx_vec2 = p.vec2[tn0 + half * (BN / 2) + row_in_tile];
       if (have_stats) {
 #pragma unroll
-        for (int j = 0; j < kStatSlots; ++j) nx_stat[j] = p.stats_in[(size_t)j * p.stats_stride + tm0 + row_in_tile];
+        for (int j = 0; j < SLOTS; ++j) nx_stat[j] = p.stats_in[(size_t)j * p.stats_stride + tm0 + row_in_tile];
       }
     };
     if (unit < tiles) request(unit);
@@ -281,7 +282,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
       if (have_stats) {
         float s = 0.0f, ss = 0.0f;
 #pragma unroll
-        for (int j = 0; j < kStatSlots; ++j) {
+        for (int j = 0; j < SLOTS; ++j) {
           s += nx_stat[j].x;
           ss += nx_stat[j].y;
         }
@@ -434,11 +435,11 @@ static int pair_mode() {
 #endif
 }
 
-template <int NC, int EPI, bool LNIN, bool STATS>
+template <int NC, int EPI, bool LNIN, bool STATS, int SLOTS>
 static int launch_variant(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tout, const CUtensorMap& tres,
                           const GemmParams& p, cudaStream_t st) {
   constexpr int kSmemBytes = smem_bytes<NC>();
-  auto kernel = gemm_tc_kernel<NC, EPI, LNIN, STATS>;
+  auto kernel = gemm_tc_kernel<NC, EPI, LNIN, STATS, SLOTS>;
   ICD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
   const int tiles = ((p.M + BM * NC - 1) / (BM * NC)) * (p.N / BN);
   int units = kSMs / NC;
@@ -469,21 +470,25 @@ static int launch_variant(const CUtensorMap& ta, const CUtensorMap& tb, const CU
   return ICD_OK;
 }
 
-template <int NC>
+// SLOTS only matters where statistics come in (LNIN, or a residual carrying them): the plain-A variants are built once
+template <int NC, int SLOTS>
 static int launch_nc(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tout, const CUtensorMap& tres,
                      const GemmParams& p, cudaStream_t st) {
   const bool lnin = p.stats_in != nullptr && p.epi != EPI_BIAS_RESIDUAL;
   const bool stats = p.stats_out != nullptr;
   switch (p.epi) {
     case EPI_BIAS:
-      return lnin ? launch_variant<NC, EPI_BIAS, true, false>(ta, tb, tout, tres, p, st)
-                  : launch_variant<NC, EPI_BIAS, false, false>(ta, tb, tout, tres, p, st);
+      return lnin ? launch_variant<NC, EPI_BIAS, true, false, SLOTS>(ta, tb, tout, tres, p, st)
+                  : launch_variant<NC, EPI_BIAS, false, false, 6>(ta, tb, tout, tres, p, st);
     case EPI_BIAS_GELU:
-      return lnin ? launch_variant<NC, EPI_BIAS_GELU, true, false>(ta, tb, tout, tres, p, st)
-                  : launch_variant<NC, EPI_BIAS_GELU, false, false>(ta, tb, tout, tres, p, st);
+      return lnin ? launch_variant<NC, EPI_BIAS_GELU, true, false, SLOTS>(ta, tb, tout, tres, p, st)
+                  : launch_variant<NC, EPI_BIAS_GELU, false, false, 6>(ta, tb, tout, tres, p, st);
     case EPI_BIAS_RESIDUAL:
-      return stats ? launch_variant<NC, EPI_BIAS_RESIDUAL, false, true>(ta, tb, tout, tres, p, st)
-                   : launch_variant<NC, EPI_BIAS_RESIDUAL, false, false>(ta, tb, tout, tres, p, st);
+      if (!p.stats_in)  // a plain residual: no statistics to add up
+        return stats ? launch_variant<NC, EPI_BIAS_RESIDUAL, false, true, 6>(ta, tb, tout, tres, p, st)
+                     : launch_variant<NC, EPI_BIAS_RESIDUAL, false, false, 6>(ta, tb, tout, tres, p, st);
+      return stats ? launch_variant<NC, EPI_BIAS_RESIDUAL, false, true, SLOTS>(ta, tb, tout, tres, p, st)
+                   : launch_variant<NC, EPI_BIAS_RESIDUAL, false, false, SLOTS>(ta, tb, tout, tres, p, st);
   }
   set_error("gemm_tc: unknown epilogue %d", p.epi);
   return ICD_E_ARG;
@@ -495,8 +500,10 @@ int launch_gemm_tc(const GemmArgs& a, cudaStream_t st) {
     return ICD_E_ARG;
   }
   if ((a.stats_in || a.stats_out) &&
-      (a.stats_stride < ((a.M + 2 * BM - 1) / (2 * BM)) * 2 * BM || (a.stats_in && (a.stats_cols != 128 * kStatSlots || !a.vec2)))) {
-    set_error("gemm_tc: LayerNorm statistics need a row stride covering whole tiles, the column vector, and a row length of 768");
+      (a.stats_stride < ((a.M + 2 * BM - 1) / (2 * BM)) * 2 * BM ||
+       (a.stats_in && ((a.stats_cols != 768 && a.stats_cols != 1024) || !a.vec2)))) {
+    set_error("gemm_tc: LayerNorm statistics need a row stride covering whole tiles, the column vector, and a row length of "
+              "768 or 1024");
     return ICD_E_ARG;
   }
   if (!a.tmap_out || (a.epi == EPI_BIAS_RESIDUAL && !a.tmap_res)) {
@@ -521,9 +528,10 @@ int launch_gemm_tc(const GemmArgs& a, cudaStream_t st) {
   p.K = a.K;
   p.epi = a.epi;
 #ifdef ICD_PROFILING
-  if (pair_mode() != 2) return launch_nc<1>(ta, tb, tout, tres, p, st);   // single-CTA tiles: A/B timing only
+  if (pair_mode() != 2)  // single-CTA tiles: A/B timing only
+    return a.stats_cols == 1024 ? launch_nc<1, 8>(ta, tb, tout, tres, p, st) : launch_nc<1, 6>(ta, tb, tout, tres, p, st);
 #endif
-  return launch_nc<2>(ta, tb, tout, tres, p, st);
+  return a.stats_cols == 1024 ? launch_nc<2, 8>(ta, tb, tout, tres, p, st) : launch_nc<2, 6>(ta, tb, tout, tres, p, st);
 }
 
 int gemm_make_map_a(void* map128, const void* base, int64_t rows, int K) {

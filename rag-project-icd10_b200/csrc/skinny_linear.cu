@@ -23,10 +23,14 @@
 //     six L2 round trips -- 3.7 us per tile and launch;
 //   * epilogue per (token, feature) as in gemm_tc.cu: bias, deferred-LayerNorm input correction, erf-GELU, residual
 //     through LayerNorm.  The row statistics the deferred LayerNorm needs are computed HERE from the rows themselves
-//     (<= 64 rows of 768), so this path neither reads nor writes the statistics buffers of the tile kernels.
+//     (<= 64 rows of H), so this path neither reads nor writes the statistics buffers of the tile kernels.
 //
-// Grid per 32 tokens: QKV 72 CTAs x 12 warps (4 feature groups x 3 K ranges), FFN-up 96 x 12, O 96 x 3, FFN-down 96 x 12;
-// at most 16 tokens: 4 warps per CTA with 768 elements of K each (launch_skinny_linear).
+// The hidden size H (768 or 1024) is a template parameter: it is the row length of those statistics, the output width
+// from which a layer counts as wide (4 feature groups per CTA) and it sets the warp budget of a CTA (12 / 16 warps).
+// Grid per 32 tokens at 768: QKV 72 CTAs x 12 warps (4 feature groups x 3 K ranges), FFN-up 96 x 12, O 96 x 3, FFN-down
+// 96 x 12; at most 16 tokens: 4 warps per CTA with 768 elements of K each (launch_skinny_linear).  At 1024: QKV 96 x 16,
+// FFN-up 128 x 16, O 128 x 4, FFN-down 128 x 16; at most 16 tokens 512 elements of K per warp (8 warps; O keeps 256), since
+// a 1024-element slice would be 128 registers of weights per lane (DESIGN.md).
 // Roofline: latency (a few microseconds per launch); the weight stream itself is ~2 us per layer at HBM speed.
 #include "common.cuh"
 #include "encoder_kernels.h"
@@ -35,10 +39,14 @@
 namespace icd {
 namespace {
 
-constexpr int kH = 768;          // hidden size: the row length every LayerNorm statistic covers
 constexpr int kMaxTokens = 64;   // rows per launch (two passes of 32)
-constexpr int kMaxWarps = 12;
 constexpr int kBlk = 8;           // 32-element K blocks per warp: a K range of 256
+// 32-element K blocks per warp when the batch is one 16-token tile (the weight slice a lane keeps in registers)
+constexpr int one_tile_blocks(int H) { return H == 768 ? 24 : 16; }
+// warps per CTA of a kernel (its launch bound): at 768 12 for every K range; at 1024 K / 256 ranges x 4 feature groups of
+// the QKV / FFN-up layers = 16 with ranges of 256 (128 registers a thread), 8 with the one-tile ranges of 512, whose
+// 64 registers of weights need the larger budget of a 256-thread CTA
+constexpr int max_warps(int H, int nblk) { return H == 768 ? 12 : (nblk == kBlk ? 16 : 8); }
 
 struct SkinnyParams {
   const __nv_bfloat16* A;    // [M, K]
@@ -69,9 +77,10 @@ __device__ __forceinline__ void mma16816(float* d, uint32_t a0, uint32_t a1, uin
 // EPI as in gemm_tc.cu; LNIN: A is an un-normalised stream (QKV of layers >= 1, FFN-up); NBLK: 32-element K blocks per warp.
 // blockIdx.y = which 32 tokens: a second pass runs on other SMs instead of after the first (one after the other, each pass
 // cost its own chain of load -> MMA -> shared-memory sum -> residual load -> store, ~2.8 us per launch: r02ai)
-template <int EPI, bool LNIN, int NBLK>
-__global__ void __launch_bounds__(32 * kMaxWarps, 1)
+template <int EPI, bool LNIN, int NBLK, int kH>
+__global__ void __launch_bounds__(32 * max_warps(kH, NBLK), 1)
 skinny_linear_kernel(const SkinnyParams p) {
+  constexpr int kMaxWarps = max_warps(kH, NBLK);
   __shared__ float s_rs[32], s_nmr[32];                    // LayerNorm of a row of this CTA's 32: y = x * rs + nmr
   const int m0 = (int)blockIdx.y * 32;
   __shared__ float s_part[kMaxWarps][2][4][32];            // K-split partial sums [warp][tile][fragment register][lane]
@@ -223,9 +232,9 @@ skinny_linear_kernel(const SkinnyParams p) {
   }
 }
 
-template <int EPI, bool LNIN, int NBLK>
+template <int EPI, bool LNIN, int NBLK, int kH>
 int launch_variant(const SkinnyParams& p, cudaStream_t st) {
-  ICD_CUDA(launch_chained(skinny_linear_kernel<EPI, LNIN, NBLK>, dim3(p.N / (8 * p.fw), (p.M + 31) / 32), dim3(32 * p.ks * p.fw), 0, st,
+  ICD_CUDA(launch_chained(skinny_linear_kernel<EPI, LNIN, NBLK, kH>, dim3(p.N / (8 * p.fw), (p.M + 31) / 32), dim3(32 * p.ks * p.fw), 0, st,
                           1, p));
   count_launch();
   return ICD_OK;
@@ -240,19 +249,56 @@ int encoder_skinny() { return g_encoder_skinny; }
 void encoder_set_skinny(int mode) { g_encoder_skinny = mode < 0 ? 0 : (mode > 2 ? 2 : mode); }
 int skinny_max_tokens() { return g_encoder_skinny == 2 ? kMaxTokens : (g_encoder_skinny == 1 ? kAutoTokens : 0); }
 
-bool skinny_linear_supported(int M, int N, int K) {
-  return M >= 1 && M <= kMaxTokens && (K == 768 || K == 3072) && N % 32 == 0 &&
-         (K / (32 * kBlk)) * (N > kH ? 4 : 1) <= kMaxWarps;
+// CTA shape of a launch: K blocks per warp, K splits and feature groups per CTA.  More than 16 tokens: K / 256 warps per
+// feature group of 8 (short K ranges keep a tile's activation loads all in flight); wide outputs (QKV, FFN-up) take four
+// groups per CTA (12 warps, 72 / 96 CTAs per 32 tokens at 768), H outputs one (O: 3 warps, FFN-down: 12; 96 CTAs).  Up to
+// 16 tokens (one tile): one warp per group over one_tile_blocks(H) * 32 elements of K (4 warps per CTA at 768, FFN-down 4 K
+// ranges) -- fewer partial sums to meet in shared memory; measured 0.337 vs 0.364 ms per 12-token forward (r02ac / r02ai),
+// and the other way round from 24 tokens on (0.49 vs 0.43).  The O projection (N = K = H) keeps K ranges of 256.
+static bool skinny_shape(int M, int N, int K, int H, int* nblk, int* ks, int* fw) {
+  if ((H != 768 && H != 1024) || M < 1 || M > kMaxTokens || N % 32 != 0) return false;
+  if (K != 768 && K != 1024 && K != 3072 && K != 4096) return false;
+  int nb = (M <= 16 && !(N == H && K == H)) ? one_tile_blocks(H) : kBlk;
+  if (K % (32 * nb) != 0) nb = kBlk;
+  *nblk = nb;
+  *ks = K / (32 * nb);
+  *fw = N > H ? 4 : 1;
+  return *ks * *fw <= max_warps(H, nb);
+}
+
+bool skinny_linear_supported(int M, int N, int K, int hidden) {
+  int nblk, ks, fw;
+  return skinny_shape(M, N, K, hidden, &nblk, &ks, &fw);
+}
+
+template <int kH, int kOne>
+static int launch_width(const SkinnyParams& p, int epi, bool lnin, int nblk, cudaStream_t st) {
+  switch (epi) {
+    case EPI_BIAS:
+      if (nblk == kOne)
+        return lnin ? launch_variant<EPI_BIAS, true, kOne, kH>(p, st) : launch_variant<EPI_BIAS, false, kOne, kH>(p, st);
+      return lnin ? launch_variant<EPI_BIAS, true, kBlk, kH>(p, st) : launch_variant<EPI_BIAS, false, kBlk, kH>(p, st);
+    case EPI_BIAS_GELU:
+      if (!lnin) break;
+      return nblk == kOne ? launch_variant<EPI_BIAS_GELU, true, kOne, kH>(p, st) : launch_variant<EPI_BIAS_GELU, true, kBlk, kH>(p, st);
+    case EPI_BIAS_RESIDUAL:
+      if (lnin) break;
+      return nblk == kOne ? launch_variant<EPI_BIAS_RESIDUAL, false, kOne, kH>(p, st)
+                          : launch_variant<EPI_BIAS_RESIDUAL, false, kBlk, kH>(p, st);
+  }
+  set_error("skinny_linear: no kernel for epilogue %d (lnin %d) at N=%d K=%d", epi, lnin ? 1 : 0, p.N, p.K);
+  return ICD_E_UNSUPPORTED;
 }
 
 int launch_skinny_linear(const SkinnyArgs& a, cudaStream_t st) {
-  if (!skinny_linear_supported(a.M, a.N, a.K)) {
-    set_error("skinny_linear: unsupported shape M=%d N=%d K=%d", a.M, a.N, a.K);
+  int nblk = 0, ks = 0, fw = 0;
+  if (!skinny_shape(a.M, a.N, a.K, a.hidden, &nblk, &ks, &fw)) {
+    set_error("skinny_linear: unsupported shape M=%d N=%d K=%d hidden=%d", a.M, a.N, a.K, a.hidden);
     return ICD_E_ARG;
   }
   const bool lnin = a.lnin != 0;
-  if ((lnin && (a.K != kH || !a.vec2)) || (a.epi == EPI_BIAS_RESIDUAL && (!a.res || (a.vec2 && a.N != kH)))) {
-    set_error("skinny_linear: LayerNorm statistics cover rows of %d elements", kH);
+  if ((lnin && (a.K != a.hidden || !a.vec2)) || (a.epi == EPI_BIAS_RESIDUAL && (!a.res || (a.vec2 && a.N != a.hidden)))) {
+    set_error("skinny_linear: LayerNorm statistics cover rows of %d elements", a.hidden);
     return ICD_E_ARG;
   }
   SkinnyParams p{};
@@ -264,30 +310,10 @@ int launch_skinny_linear(const SkinnyArgs& a, cudaStream_t st) {
   p.out = reinterpret_cast<__nv_bfloat16*>(a.out);
   p.M = a.M, p.N = a.N, p.K = a.K;
   p.eps = a.eps;
-  // shape of a CTA.  More than 16 tokens: K / 256 warps per feature group of 8 (short K ranges keep a tile's activation
-  // loads all in flight); wide outputs (QKV, FFN-up) take four groups per CTA (12 warps, 72 / 96 CTAs per 32 tokens),
-  // 768 outputs one (O: 3 warps, FFN-down: 12; 96 CTAs).  Up to 16 tokens (one tile): one warp per group over 768
-  // elements of K (4 warps per CTA, FFN-down 4 K ranges) -- fewer partial sums to meet in shared memory; measured 0.337 vs
-  // 0.364 ms per 12-token forward (r02ac / r02ai), and the other way round from 24 tokens on (0.49 vs 0.43).
-  const bool one_tile = a.M <= 16;
-  const int nblk = (one_tile && !(a.N == kH && a.K == kH)) ? 24 : kBlk;
-  p.ks = a.K / (32 * nblk);
-  p.fw = a.N > kH ? 4 : 1;
-  if (p.ks * p.fw <= kMaxWarps) {
-    switch (a.epi) {
-      case EPI_BIAS:
-        if (nblk == 24) return lnin ? launch_variant<EPI_BIAS, true, 24>(p, st) : launch_variant<EPI_BIAS, false, 24>(p, st);
-        return lnin ? launch_variant<EPI_BIAS, true, kBlk>(p, st) : launch_variant<EPI_BIAS, false, kBlk>(p, st);
-      case EPI_BIAS_GELU:
-        if (!lnin) break;
-        return nblk == 24 ? launch_variant<EPI_BIAS_GELU, true, 24>(p, st) : launch_variant<EPI_BIAS_GELU, true, kBlk>(p, st);
-      case EPI_BIAS_RESIDUAL:
-        if (lnin) break;
-        return nblk == 24 ? launch_variant<EPI_BIAS_RESIDUAL, false, 24>(p, st) : launch_variant<EPI_BIAS_RESIDUAL, false, kBlk>(p, st);
-    }
-  }
-  set_error("skinny_linear: no kernel for epilogue %d (lnin %d) at N=%d K=%d", a.epi, a.lnin, a.N, a.K);
-  return ICD_E_UNSUPPORTED;
+  p.ks = ks;
+  p.fw = fw;
+  return a.hidden == 768 ? launch_width<768, one_tile_blocks(768)>(p, a.epi, lnin, nblk, st)
+                         : launch_width<1024, one_tile_blocks(1024)>(p, a.epi, lnin, nblk, st);
 }
 
 }  // namespace icd

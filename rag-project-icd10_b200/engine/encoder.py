@@ -19,7 +19,7 @@ from .. import _native as N
 from . import weights as W
 from .tokenizer import NativeTokenizer
 
-MAX_S = 512  # kernel limit (BERT's position table); text2vec-base-chinese's own max_seq_length is 128
+MAX_S = 512  # kernel limit (BERT's position table); text2vec-base-chinese's own max_seq_length is 128, e5-large's 512
 FEED_CHUNK = 32768   # sentences tokenised / length-bucketed / copied back as one unit of the feeder pipeline
 SMALL_BATCH = 256    # up to this many sentences take the direct path (one tokeniser call, synchronous launches)
 
@@ -28,20 +28,27 @@ class EncoderEngine:
     def __init__(self, model_name_or_path: Optional[str] = None, device: Union[str, int, None] = None, *,
                  cfg: Optional[N.BertCfg] = None, blob: Optional[np.ndarray] = None, tokenizer=None,
                  max_seq_length: int = 128, max_tokens: int = 4096 * 64, vocab_path: Optional[str] = None,
-                 host_threads: Optional[int] = None):
+                 host_threads: Optional[int] = None, position_offset: int = 0, unk_id: Optional[int] = None):
+        """position_offset / unk_id (programmatic use with cfg= / blob=; a model directory supplies its own): token t
+        of a sequence reads position row position_offset + t (XLM-R: pad_token_id + 1), ids outside the vocabulary
+        read row unk_id (None: [UNK] = 100 of BERT vocabularies)."""
         N.require_gpu()
         self.device_index = _device_index(device)
         if blob is None:
             path = W.resolve_model_dir(model_name_or_path)
             cfg, blob, meta = W.load_model_dir(path)
             max_seq_length = meta["max_seq_length"]
+            position_offset, unk_id = meta["position_offset"], meta["unk_id"]
             if tokenizer is None:
                 tokenizer = load_tokenizer(path)
         if tokenizer is None:
             raise ValueError("a tokenizer is required")
         self.cfg = cfg
         self.tokenizer = tokenizer
-        self.max_seq_length = min(int(max_seq_length), MAX_S, cfg.max_position)
+        self.position_offset = int(position_offset)
+        self.unk_id = unk_id
+        # position rows position_offset .. position_offset + S - 1 must exist (XLM-R: 514 rows, offset 2 -> 512 tokens)
+        self.max_seq_length = min(int(max_seq_length), MAX_S, cfg.max_position - self.position_offset)
         self.max_tokens = int(max_tokens)
         self.vocab_path = vocab_path
         self.last_stats: dict = {}
@@ -55,6 +62,8 @@ class EncoderEngine:
         blob = np.ascontiguousarray(blob, np.float32)
         N.check(N.lib().icd_encoder_create(N.buf_ptr(blob), blob.size, C.byref(cfg), self.device_index,
                                            C.byref(self._h)), "icd_encoder_create")
+        N.check(N.lib().icd_encoder_set_embedding_ids(self._h, self.position_offset, -1 if unk_id is None else int(unk_id)),
+                "icd_encoder_set_embedding_ids")
 
     # ---------------------------------------------------------------- SentenceTransformer surface
     def get_sentence_embedding_dimension(self) -> int:

@@ -116,6 +116,9 @@ class TokenClassifierEngine:
         if encoder is None:
             path = W.resolve_model_dir(model_name_or_path, allow_env_override=False)
             cfg, blob, _meta = W.load_model_dir(path)
+            if _meta["position_offset"]:
+                raise ValueError(f"{path}: token classification is served for BERT models only (XLM-RoBERTa position "
+                                 "numbering is supported by the sentence encoder)")
             state = W.load_state(path)
             head_weight = np.asarray(state["classifier.weight"], np.float32)
             head_bias = np.asarray(state["classifier.bias"], np.float32)

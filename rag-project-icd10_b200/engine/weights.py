@@ -1,29 +1,44 @@
 """Weight blob for icd_encoder_create: HF BertModel tensors flattened to fp32 in the canonical
 order documented in csrc/api_encoder.cu.  Loads an HF / sentence-transformers model directory
-(config.json + model.safetensors | pytorch_model.bin + vocab.txt), the layout
+(config.json + model.safetensors | pytorch_model.bin + vocab.txt | tokenizer.json), the layout
 SentenceTransformer(model_name) resolves in the reference (services/embedding_service.py:61).
+
+Two encoder shapes are served: hidden 768 with 12 heads (BERT-base, text2vec-base-chinese) and hidden 1024 with 16
+heads (BERT-large, XLM-RoBERTa-large: intfloat/multilingual-e5-large(-instruct), the reference's code default).
+XLMRobertaModel has BertModel's tensors and arithmetic; it differs in two embedding conventions, which `meta` carries:
+positions of real tokens start at pad_token_id + 1, and <unk> is id 3.
 """
 from __future__ import annotations
 
 import json
 import os
-from typing import Dict, Tuple
+from typing import Dict, Optional, Tuple
 
 import numpy as np
 
 from .. import _native as N
 
 
+MODEL_TYPES = ("bert", "xlm-roberta")
+SHAPES = {768: 12, 1024: 16}      # hidden size -> attention heads (head dim 64)
+
+
 def config_from_dict(cfg: dict) -> N.BertCfg:
-    if cfg.get("model_type", "bert") != "bert":
-        raise ValueError(f"only BERT-base encoders are supported (model_type={cfg.get('model_type')}); the supported "
-                         "embedding model is shibing624/text2vec-base-chinese (EMBEDDING_MODEL_NAME in the reference's "
-                         "env.example) -- the reference's code default intfloat/multilingual-e5-large-instruct is XLM-R "
-                         "large and is not served by this engine")
+    mt = cfg.get("model_type", "bert")
+    if mt not in MODEL_TYPES:
+        raise ValueError(f"model_type {mt!r} is not supported: BERT and XLM-RoBERTa encoders only (hidden 768 / 12 heads "
+                         "or 1024 / 16 heads)")
     if cfg.get("hidden_act", "gelu") != "gelu":
         raise ValueError("only erf-GELU ('gelu') is supported")
     if cfg.get("position_embedding_type", "absolute") != "absolute":
         raise ValueError("only absolute position embeddings are supported")
+    hidden, heads = int(cfg["hidden_size"]), int(cfg["num_attention_heads"])
+    if heads * 64 != hidden:
+        raise ValueError(f"head dim must be 64: hidden {hidden} with {heads} heads is not supported (supported shapes: "
+                         "hidden 768 with 12 heads, hidden 1024 with 16 heads)")
+    if hidden not in SHAPES:
+        raise ValueError(f"hidden size {hidden} is not supported (supported shapes: hidden 768 with 12 heads, hidden 1024 "
+                         "with 16 heads)")
     return N.BertCfg(vocab_size=int(cfg["vocab_size"]), hidden=int(cfg["hidden_size"]),
                      layers=int(cfg["num_hidden_layers"]), heads=int(cfg["num_attention_heads"]),
                      intermediate=int(cfg["intermediate_size"]), max_position=int(cfg["max_position_embeddings"]),
@@ -46,9 +61,10 @@ def tensor_order(layers: int):
 
 
 def pack_state_dict(state: Dict[str, "np.ndarray"], cfg: N.BertCfg) -> np.ndarray:
-    """state: name -> array-like (torch tensors accepted); names may carry a 'bert.' prefix."""
+    """state: name -> array-like (torch tensors accepted); names may carry a 'bert.', 'roberta.' or '0.auto_model.'
+    prefix."""
     def get(name):
-        for cand in (name, "bert." + name, "0.auto_model." + name):
+        for cand in (name, "bert." + name, "roberta." + name, "0.auto_model." + name):
             if cand in state:
                 t = state[cand]
                 if hasattr(t, "detach"):
@@ -90,12 +106,43 @@ def load_state(path: str) -> dict:
     return {k: v.float().numpy() for k, v in state.items()}
 
 
+def position_offset(cfg: dict) -> int:
+    """First position row of a sequence's real tokens: XLM-R numbers them from pad_token_id + 1 (create_position_ids_
+    from_input_ids on a right-padded batch), BERT from 0."""
+    if cfg.get("model_type", "bert") == "xlm-roberta":
+        return int(cfg.get("pad_token_id", 1)) + 1
+    return 0
+
+
+def unk_id(path: str) -> Optional[int]:
+    """The unknown-token id of the directory's tokenizer (tokenizer.json, else vocab.txt); None if neither says."""
+    tj = os.path.join(path, "tokenizer.json")
+    if os.path.exists(tj):
+        with open(tj, encoding="utf-8") as fh:
+            model = json.load(fh).get("model") or {}
+        if model.get("type") == "Unigram" and model.get("unk_id") is not None:
+            return int(model["unk_id"])
+        vocab = model.get("vocab")
+        if isinstance(vocab, dict) and model.get("unk_token") in vocab:
+            return int(vocab[model["unk_token"]])
+    vt = os.path.join(path, "vocab.txt")
+    if os.path.exists(vt):
+        with open(vt, encoding="utf-8") as fh:
+            for i, line in enumerate(fh):
+                if line.rstrip("\n") == "[UNK]":
+                    return i
+    return None
+
+
 def load_model_dir(path: str) -> Tuple[N.BertCfg, np.ndarray, dict]:
+    """(config, weight blob, meta); meta: max_seq_length, do_lower_case_text, pooling, position_offset, unk_id (None:
+    the library's default rule)."""
     with open(os.path.join(path, "config.json"), encoding="utf-8") as fh:
         cfg_d = json.load(fh)
     cfg = config_from_dict(cfg_d)
     state = load_state(path)
-    meta = {"max_seq_length": 128, "do_lower_case_text": False, "pooling": "mean"}
+    meta = {"max_seq_length": 128, "do_lower_case_text": False, "pooling": "mean",
+            "position_offset": position_offset(cfg_d), "unk_id": unk_id(path)}
     sb = os.path.join(path, "sentence_bert_config.json")
     if os.path.exists(sb):
         with open(sb, encoding="utf-8") as fh:
