@@ -140,6 +140,9 @@ int icd_index_set_timing(icd_index* idx, int enabled);   /* also restarts the ca
  * (the most recent 64 of them); *calls = how many were averaged.  Synchronises with the last one only,
  * so a timed region of back-to-back searches is measured without host syncs in between. */
 int icd_index_mean_timing(const icd_index* idx, float* us3, int* calls);
+/* queries the tensor path could not certify exact and re-searched with the exact stream scan since the previous call
+ * (waits for the device); the counter restarts at 0 */
+int icd_index_take_fallbacks(icd_index* idx, int64_t* count);
 
 /* ---------------------------------------------------------------- row-sharded scan ---------
  * New work (the reference is single-process): rank r holds rows [row_offset, row_offset+n_r);

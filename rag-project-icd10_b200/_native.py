@@ -28,7 +28,7 @@ SYMBOLS = [
     "icd_version", "icd_last_error", "icd_launch_count", "icd_device_count", "icd_tune",
     "icd_index_create", "icd_index_destroy", "icd_index_append", "icd_index_adopt", "icd_index_clear",
     "icd_index_size", "icd_index_dim", "icd_index_read", "icd_index_search", "icd_index_last_timing",
-    "icd_index_set_timing", "icd_index_mean_timing", "icd_index_search_filtered",
+    "icd_index_set_timing", "icd_index_mean_timing", "icd_index_search_filtered", "icd_index_take_fallbacks",
     "icd_nccl_unique_id", "icd_shard_group_create", "icd_shard_group_destroy",
     "icd_shard_group_export_slab", "icd_shard_group_import_slabs", "icd_shard_group_search",
     "icd_shard_group_search_filtered",
@@ -115,6 +115,7 @@ def _declare(L: C.CDLL) -> None:
     L.icd_index_last_timing.argtypes = [vp, f32p, C.POINTER(i32)]
     L.icd_index_set_timing.argtypes = [vp, i32]
     L.icd_index_mean_timing.argtypes = [vp, f32p, C.POINTER(i32)]
+    L.icd_index_take_fallbacks.argtypes = [vp, C.POINTER(i64)]
     if hasattr(L, "icd_nccl_unique_id"):
         L.icd_nccl_unique_id.argtypes = [vp]
         L.icd_shard_group_create.argtypes = [vp, i32, i32, i64, vp, C.POINTER(vp)]

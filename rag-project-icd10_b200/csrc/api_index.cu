@@ -103,6 +103,11 @@ int index_search_device(icd_index* x, int B, int k, int weight_mode, int path, i
   }
   const bool scan_f32rows = !use_tc && have_master;
   const bool rescore_f32rows = have_master;
+  // Where the tensor scan's scores are not the canonical products (fp32 master rows, or fp32 queries rounded to bf16)
+  // its top-kc need not hold the exact top-k: finalise certifies each query and the exact stream scan re-searches the
+  // others.  bf16 queries on bf16 rows score the canonical products themselves, and the k + 6 margin covers the fp32
+  // accumulation order (DESIGN.md, "Exact search").
+  const bool certify = use_tc && n > 0 && (have_master || !q_exact_bf16);
 
   // candidates per query kept by the scan
   int kc = k;
@@ -112,6 +117,10 @@ int index_search_device(icd_index* x, int B, int k, int weight_mode, int path, i
   const int P = use_tc ? tensor_scan_max_partials() : stream_scan_grid();
   ICD_TRY(x->part_score.reserve((size_t)B * P * std::max(kc, use_tc ? tensor_scan_pre_slots() : kc) * 4));
   ICD_TRY(x->part_id.reserve((size_t)B * P * kc * 4));
+  if (certify) {
+    ICD_TRY(x->part_score.reserve((size_t)B * stream_scan_grid() * k * 4));
+    ICD_TRY(x->part_id.reserve((size_t)B * stream_scan_grid() * k * 4));
+  }
   ICD_TRY(x->cand_score.reserve((size_t)B * kc * 4));
   ICD_TRY(x->cand_id.reserve((size_t)B * kc * 8));
 
@@ -251,7 +260,49 @@ int index_search_device(icd_index* x, int B, int k, int weight_mode, int path, i
   f.out_id = d_id;
   f.out_level = d_level;
   if (push) f.push = *push;
+  if (certify) {
+    ICD_CUDA(cudaMemsetAsync(x->fb.ptr, 0, 4, st));
+    f.colstat = (const float*)x->colstat.ptr;
+    f.fb = (int*)x->fb.ptr;
+  }
   ICD_TRY(launch_finalise(f, st));
+  if (certify) {
+    // exact fallback for the uncertified queries, listed on the device: stream scan (one query per pass), merge and
+    // finalise of list slot j into query fb[2 + j]'s result rows (and pushes, so a shard exchange sees only exact blocks)
+    const int* fb = (const int*)x->fb.ptr;
+    StreamScanArgs s{};
+    s.table = have_master ? (const void*)x->master : (const void*)x->table;
+    s.levels = x->levels;
+    s.n_rows = n;
+    s.dim = x->dim;
+    s.f32rows = have_master;
+    s.q = (const float*)x->q_f32.ptr;
+    s.nq = B;
+    s.k = k;
+    s.weight_pre = weight_pre;
+    s.part_score = (float*)x->part_score.ptr;
+    s.part_id = (int*)x->part_id.ptr;
+    s.P = stream_scan_grid();
+    s.mask = d_mask;
+    ICD_TRY(launch_stream_scan_listed(s, fb, st));
+    MergeArgs m{};
+    m.part_score = (const float*)x->part_score.ptr;
+    m.part_id = (const int*)x->part_id.ptr;
+    m.B = B;
+    m.P = s.P;
+    m.k_in = k;
+    m.k_out = k;
+    m.out_score = (float*)x->cand_score.ptr;
+    m.out_id = (int64_t*)x->cand_id.ptr;
+    m.row_offset = row_offset;
+    m.count = fb;
+    ICD_TRY(launch_merge(m, st));
+    f.kcp = k;
+    f.colstat = nullptr;
+    f.fb = nullptr;
+    f.fb_in = fb;
+    ICD_TRY(launch_finalise(f, st));
+  }
   if (x->timing) cudaEventRecord(ev[3], st);
   x->last_launches = (int)(g_launches.load() - l0);
   x->timing_pending = x->timing;
@@ -358,7 +409,19 @@ int icd_index_create(int dim, int device, int64_t capacity_rows, int flags, icd_
   x->device = device;
   x->flags = flags;
   int st = alloc_table(x, std::max<int64_t>(capacity_rows, 1024));
+  if (st == ICD_OK) st = x->colstat.reserve((size_t)(2 * dim + 2) * 4);
+  if (st == ICD_OK) st = x->fb.reserve((size_t)(2 + 8192) * 4);
+  if (st == ICD_OK && (cudaMemset(x->colstat.ptr, 0, (size_t)(2 * dim + 2) * 4) != cudaSuccess ||
+                       cudaMemset(x->fb.ptr, 0, 8) != cudaSuccess)) {
+    set_error("icd_index_create: cudaMemset failed");
+    st = ICD_E_CUDA;
+  }
   if (st != ICD_OK) {
+    if (x->table) cudaFree(x->table);
+    if (x->master) cudaFree(x->master);
+    if (x->levels) cudaFree(x->levels);
+    x->colstat.release();
+    x->fb.release();
     delete x;
     return st;
   }
@@ -387,6 +450,8 @@ int icd_index_destroy(icd_index* x) {
   x->in_stage.release();
   x->gbound.release();
   x->mask.release();
+  x->colstat.release();
+  x->fb.release();
   x->q_f32_alt.release();
   x->q_bf16_alt.release();
   x->out_stage_alt.release();
@@ -439,6 +504,7 @@ int icd_index_append(icd_index* x, const void* vecs, int dtype, const uint8_t* l
   } else {
     ICD_CUDA(cudaMemsetAsync(x->levels + x->n, 1, n, st));
   }
+  ICD_TRY(launch_column_stats(x->table, x->master, x->n, n, x->dim, (float*)x->colstat.ptr, st));
   ICD_CUDA(cudaStreamSynchronize(st));
   x->n += n;
   x->map_valid = false;
@@ -466,6 +532,9 @@ int icd_index_adopt(icd_index* x, const void* dev_bf16, const uint8_t* dev_level
   x->n = n;
   x->cap = n;
   x->map_valid = false;
+  ICD_CUDA(cudaMemset(x->colstat.ptr, 0, (size_t)(2 * x->dim + 2) * 4));
+  ICD_TRY(launch_column_stats(x->table, nullptr, 0, n, x->dim, (float*)x->colstat.ptr, 0));
+  ICD_CUDA(cudaStreamSynchronize(0));
   return ICD_OK;
 }
 
@@ -477,6 +546,19 @@ int icd_index_clear(icd_index* x) {
   }
   x->n = 0;
   x->map_valid = false;
+  DeviceGuard g(x->device);
+  ICD_CUDA(cudaMemset(x->colstat.ptr, 0, (size_t)(2 * x->dim + 2) * 4));
+  return ICD_OK;
+}
+
+int icd_index_take_fallbacks(icd_index* x, int64_t* count) {
+  ICD_CHECK_ARG(x != nullptr && count != nullptr, "null argument");
+  DeviceGuard g(x->device);
+  int v = 0;
+  ICD_CUDA(cudaDeviceSynchronize());
+  ICD_CUDA(cudaMemcpy(&v, (const int*)x->fb.ptr + 1, 4, cudaMemcpyDeviceToHost));
+  ICD_CUDA(cudaMemset((int*)x->fb.ptr + 1, 0, 4));
+  *count = v;
   return ICD_OK;
 }
 

@@ -34,6 +34,9 @@ struct icd_index {
   // workspace
   icd::DeviceBuf q_f32, q_bf16, part_score, part_id, cand_score, cand_id, out_stage, in_stage, gbound;
   icd::DeviceBuf mask;   // a row mask handed over in host memory, copied in like the queries
+  // exactness certificate of the tensor path: [2][dim] column maxima and 2 row-norm maxima (launch_column_stats), the list of
+  // queries it could not certify: [count of this search, total since icd_index_take_fallbacks, query ids (<= 8192)]
+  icd::DeviceBuf colstat, fb;
   // pipelined searches from host buffers (icd_index_search, large batches): the second set of query / result staging
   // buffers, the copy stream and the events that order the two streams
   icd::DeviceBuf q_f32_alt, q_bf16_alt, out_stage_alt;

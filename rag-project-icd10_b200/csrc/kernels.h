@@ -25,6 +25,10 @@ struct StreamScanArgs {
 int stream_scan_grid();
 int stream_scan_max_queries(bool f32rows, int dim);
 int launch_stream_scan(const StreamScanArgs& a, cudaStream_t st);
+// exact fallback of the tensor path: one query per pass over the queries listed in device memory (fb = [count, total,
+// query ids...] as finalise_kernel leaves it); a.q is the whole batch [B, dim], a.nq = B bounds the list, slot j of the
+// list writes partial row j.  The count stays on the device, so the call does not synchronise.
+int launch_stream_scan_listed(const StreamScanArgs& a, const int* fb, cudaStream_t st);
 
 // ---- scan_tc.cu (tcgen05 / TMEM / TMA)
 struct TensorScanArgs {
@@ -73,6 +77,7 @@ struct MergeArgs {
   int64_t row_offset;
   int* bound_key_out;        // [B] or null: order-preserving key of the k_out-th score (very negative when
                              // the list holds fewer than k_out rows) -- the admission bound of the main scan
+  const int* count;          // or null: only the first *count of the B lists are live (the exact fallback's)
 };
 int launch_merge(const MergeArgs& a, cudaStream_t st);
 // pre-pass bound: per query the kc-th largest of the slot maxima (each slot's maximum taken over the row groups of one
@@ -120,11 +125,22 @@ struct FinaliseArgs {
   // fused exchange, consumer side: CTA b waits for wait_flag[s][b] == epoch of every source
   const uint32_t* wait_flag;  // [S][B] or null
   uint32_t epoch;
+  // Exactness certificate of the tensor path (colstat != null, S == 1): cand_score holds the scan's own scores, and a
+  // query is certified when its k-th canonical key beats the kc-th scan score by more than the scan's error bound
+  // (DESIGN.md, "Exact search").  An uncertified query writes nothing and appends its id to fb = [count, total, ids...].
+  const float* colstat;  // [2][dim]: max |row_i| (bf16 image and master), max |master_i - bf16(master_i)|; then the
+                         // largest row norm (either copy) and the largest |master row - bf16 row|
+  int* fb;
+  // the fallback's finalise: CTA j serves query fb_in[2 + j] if j < fb_in[0], its candidates in row j of cand_*
+  const int* fb_in;
 };
 int launch_finalise(const FinaliseArgs& a, cudaStream_t st);
 
 // elementwise helpers
 int launch_f32_to_bf16(const float* in, void* out_bf16, int64_t n, cudaStream_t st);
 int launch_bf16_to_f32(const void* in_bf16, float* out, int64_t n, cudaStream_t st);
+// per-column maxima of rows [row0, row0 + n) folded into colstat (see FinaliseArgs::colstat); master may be null
+int launch_column_stats(const void* table_bf16, const float* master, int64_t row0, int64_t n, int dim, float* colstat,
+                        cudaStream_t st);
 
 }  // namespace icd

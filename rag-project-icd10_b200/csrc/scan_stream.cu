@@ -89,11 +89,11 @@ __device__ __forceinline__ float warp_list_insert(float* sc, int* id, int k, flo
 // set in `mask` are read and inserted (a template parameter: the widest variants have no register to spare, so the
 // unfiltered scan stays exactly what it was).
 template <int NQ, int CPL, bool F32ROWS, int R, bool MASKED>
-__global__ void __launch_bounds__(kWarps * 32, 2)
-scan_stream_kernel(const void* __restrict__ table, const uint8_t* __restrict__ levels, int64_t n_rows,
-                   int dim, const float* __restrict__ q, int nq_valid, int k, int weight_pre,
-                   float* __restrict__ part_score, int* __restrict__ part_id, int q0, int P,
-                   const uint32_t* __restrict__ mask) {
+__device__ __forceinline__ void scan_stream_body(const void* __restrict__ table, const uint8_t* __restrict__ levels,
+                                                 int64_t n_rows, int dim, const float* __restrict__ q, int nq_valid,
+                                                 int k, int weight_pre, float* __restrict__ part_score,
+                                                 int* __restrict__ part_id, int q0, int P,
+                                                 const uint32_t* __restrict__ mask) {
   constexpr int E = RowChunk<F32ROWS>::kElems;
   constexpr int kRowsPerWarpIter = R;
   constexpr int kRowsPerCtaIter = kWarps * R;
@@ -218,6 +218,33 @@ scan_stream_kernel(const void* __restrict__ table, const uint8_t* __restrict__ l
   }
 }
 
+template <int NQ, int CPL, bool F32ROWS, int R, bool MASKED>
+__global__ void __launch_bounds__(kWarps * 32, 2)
+scan_stream_kernel(const void* __restrict__ table, const uint8_t* __restrict__ levels, int64_t n_rows,
+                   int dim, const float* __restrict__ q, int nq_valid, int k, int weight_pre,
+                   float* __restrict__ part_score, int* __restrict__ part_id, int q0, int P,
+                   const uint32_t* __restrict__ mask) {
+  scan_stream_body<NQ, CPL, F32ROWS, R, MASKED>(table, levels, n_rows, dim, q, nq_valid, k, weight_pre, part_score,
+                                                part_id, q0, P, mask);
+}
+
+// The tensor path's exact fallback: the queries listed in fb[2 ..] (fb[0] of them, at most nq_max), one per pass; grid.y
+// slots walk the list, slot j's partial lists go to row j of the partial buffer.
+template <int CPL, bool F32ROWS, int R, bool MASKED>
+__global__ void __launch_bounds__(kWarps * 32, 2)
+scan_stream_listed_kernel(const void* __restrict__ table, const uint8_t* __restrict__ levels, int64_t n_rows,
+                          int dim, const float* __restrict__ q, int nq_max, int k, int weight_pre,
+                          float* __restrict__ part_score, int* __restrict__ part_id, int P,
+                          const uint32_t* __restrict__ mask, const int* __restrict__ fb) {
+  const int count = min(fb[0], nq_max);
+  for (int j = blockIdx.y; j < count; j += gridDim.y) {
+    const float* qj = q + (size_t)fb[2 + j] * dim;
+    scan_stream_body<1, CPL, F32ROWS, R, MASKED>(table, levels, n_rows, dim, qj, 1, k, weight_pre, part_score, part_id,
+                                                 j, P, mask);
+    __syncthreads();   // the next pass re-initialises the lists this pass's merge reads
+  }
+}
+
 template <int NQ, int CPL, bool F32ROWS, int R>
 int launch_one(const StreamScanArgs& a, int grid, size_t smem, cudaStream_t st) {
   auto kern = a.mask ? scan_stream_kernel<NQ, CPL, F32ROWS, R, true> : scan_stream_kernel<NQ, CPL, F32ROWS, R, false>;
@@ -265,7 +292,45 @@ int launch_f32(const StreamScanArgs& a, int grid, size_t smem, cudaStream_t st) 
   return ICD_E_UNSUPPORTED;
 }
 
+template <int CPL, bool F32ROWS, int R>
+int launch_listed_one(const StreamScanArgs& a, const int* fb, size_t smem, cudaStream_t st) {
+  auto kern = a.mask ? scan_stream_listed_kernel<CPL, F32ROWS, R, true> : scan_stream_listed_kernel<CPL, F32ROWS, R, false>;
+  ICD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  // 8 list slots in flight: a handful of uncertified queries costs one pass over the table, and a CTA whose slots are
+  // past the count exits at once
+  const dim3 grid(a.P, std::min(a.nq, 8));
+  kern<<<grid, kWarps * 32, smem, st>>>(a.table, a.levels, a.n_rows, a.dim, a.q, a.nq, a.k, a.weight_pre, a.part_score,
+                                        a.part_id, a.P, a.mask, fb);
+  count_launch();
+  ICD_CUDA(cudaGetLastError());
+  return ICD_OK;
+}
+
 }  // namespace
+
+int launch_stream_scan_listed(const StreamScanArgs& a, const int* fb, cudaStream_t st) {
+  const size_t smem = (size_t)kWarps * a.k * 8;
+  if (a.f32rows) {
+    switch ((a.dim / 4 + 31) / 32) {
+      case 1: return launch_listed_one<1, true, 4>(a, fb, smem, st);
+      case 2: return launch_listed_one<2, true, 4>(a, fb, smem, st);
+      case 3: return launch_listed_one<3, true, 2>(a, fb, smem, st);
+      case 4: return launch_listed_one<4, true, 2>(a, fb, smem, st);
+      case 5:
+      case 6: return launch_listed_one<6, true, 2>(a, fb, smem, st);
+      default: break;
+    }
+  } else {
+    switch ((a.dim / 8 + 31) / 32) {
+      case 1: return launch_listed_one<1, false, 4>(a, fb, smem, st);
+      case 2: return launch_listed_one<2, false, 4>(a, fb, smem, st);
+      case 3: return launch_listed_one<3, false, 4>(a, fb, smem, st);
+      default: break;
+    }
+  }
+  set_error("scan_stream: no listed variant for dim %d (the tensor path serves dim <= 768)", a.dim);
+  return ICD_E_UNSUPPORTED;
+}
 
 int stream_scan_grid() { return kSMs * 2; }
 int stream_scan_max_queries(bool f32rows, int dim) { return f32rows ? 1 : (dim > 768 ? 2 : 4); }

@@ -16,11 +16,11 @@ constexpr int kMaxP = 1024;
 __global__ void __launch_bounds__(kMergeWarps * 32)
 merge_kernel(const float* __restrict__ part_score, const int* __restrict__ part_id, int B, int P,
              int k_in, int k_out, float* __restrict__ out_score, int64_t* __restrict__ out_id,
-             int64_t row_offset, int* __restrict__ bound_key_out) {
+             int64_t row_offset, int* __restrict__ bound_key_out, const int* __restrict__ count) {
   __shared__ unsigned char heads[kMergeWarps][kMaxP];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x * kMergeWarps + warp;
-  if (b >= B) return;
+  if (b >= B || (count && b >= *count)) return;
   unsigned char* hd = heads[warp];
   for (int l = lane; l < P; l += 32) hd[l] = 0;
   __syncwarp();
@@ -154,10 +154,20 @@ finalise_kernel(FinaliseArgs a) {
   __shared__ int64_t s_id[kMaxCand];
   __shared__ uint8_t s_lv[kMaxCand];
   __shared__ float t_raw[ICD_MAX_K];
+  __shared__ float t_key[ICD_MAX_K];
   __shared__ double t_w[ICD_MAX_K];
+  constexpr int kRed = 8;
+  __shared__ double s_red[kRed][kFinThreads / 32];
+  __shared__ int s_certified;
   __shared__ int64_t t_id[ICD_MAX_K];
   __shared__ uint8_t t_lv[ICD_MAX_K];
-  const int b = blockIdx.x;
+  // cb: this CTA's row of the candidate arrays; b: its query (they differ in the exact fallback's finalise)
+  const int cb = blockIdx.x;
+  int b = blockIdx.x;
+  if (a.fb_in) {
+    if (cb >= a.fb_in[0]) return;
+    b = a.fb_in[2 + cb];
+  }
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int kc = a.S * a.kcp;
 
@@ -188,12 +198,12 @@ finalise_kernel(FinaliseArgs a) {
   //    trips per candidate, nine candidates per warp in a row: 27 - 40 us per launch at small batches, r02w)
   for (int c = threadIdx.x; c < kc; c += kFinThreads) {
     const int s = c / a.kcp, j = c % a.kcp;
-    size_t src = ((size_t)s * a.B + b) * a.kcp + j;
+    size_t src = ((size_t)s * a.B + cb) * a.kcp + j;
     const float* cs = a.cand_score;
     const int64_t* ci = a.cand_id;
     const uint8_t* cl = a.cand_level;
     if (a.src_stride_bytes) {
-      src = (size_t)b * a.kcp + j;
+      src = (size_t)cb * a.kcp + j;
       cs = reinterpret_cast<const float*>(reinterpret_cast<const char*>(cs) + (size_t)s * a.src_stride_bytes);
       ci = reinterpret_cast<const int64_t*>(reinterpret_cast<const char*>(ci) + (size_t)s * a.src_stride_bytes);
       if (cl) cl += (size_t)s * a.src_stride_bytes;
@@ -249,6 +259,7 @@ finalise_kernel(FinaliseArgs a) {
     }
     if (rank < a.k) {
       t_raw[rank] = s_raw[c];
+      t_key[rank] = kc_s;
       t_id[rank] = kc_i;
       t_lv[rank] = s_lv[c];
       t_w[rank] = (kc_i < 0) ? -INFINITY
@@ -258,6 +269,66 @@ finalise_kernel(FinaliseArgs a) {
   }
   __syncthreads();
   const int kk = min(a.k, kc);
+
+  // 2b. exactness certificate of the tensor path.  Every row outside the candidates has a scan score <= s_kc, the
+  //     kc-th candidate's (the scan keeps its top kc, and its pruning bound never exceeds that score).  A row's canonical
+  //     score differs from its scan score by at most A (rounding the query to bf16, and the master rows to the bf16
+  //     image the scan reads) + T (tensor-core fp32 accumulation, 2 K 2^-24 of the absolute products) + C (the canonical
+  //     dot, (L + 5) 2^-24 of them), each bounded per query through the column maxima.  If the k-th returned key beats
+  //     s_kc by more than that slack (times the largest level weight under WEIGHT_PRE), no outside row can enter the
+  //     top k; otherwise the query is listed for the exact stream scan and writes nothing here.
+  if (a.colstat) {
+    // each term bounded two ways, through the column maxima and (Cauchy-Schwarz) through the largest row norms
+    double r[kRed] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    const float* qv = a.q_f32 + (size_t)b * a.dim;
+    for (int i = threadIdx.x; i < a.dim; i += kFinThreads) {
+      const double qi = qv[i];
+      const double bq = (double)__bfloat162float(__float2bfloat16_rn(qv[i]));
+      const double M = a.colstat[i], D = a.colstat[a.dim + i];
+      r[0] += fabs(qi - bq) * M;
+      r[1] += fabs(bq) * D;
+      r[2] += fabs(bq) * M;
+      r[3] += fabs(qi) * (M + D);
+      r[4] += (qi - bq) * (qi - bq);
+      r[5] += bq * bq;
+      r[6] += qi * qi;
+    }
+#pragma unroll
+    for (int j = 0; j < kRed; ++j) {
+#pragma unroll
+      for (int off = 16; off > 0; off >>= 1) r[j] += __shfl_xor_sync(0xffffffffu, r[j], off);
+      if (lane == 0) s_red[j][warp] = r[j];
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      double t[kRed] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+      for (int j = 0; j < kRed; ++j)
+        for (int w = 0; w < kFinThreads / 32; ++w) t[j] += s_red[j][w];
+      const double R = a.colstat[2 * a.dim], Rd = a.colstat[2 * a.dim + 1];   // max row norms: rows, master - bf16
+      const double nd = sqrt(t[4]) * (1.0 + 1e-6), nb = sqrt(t[5]) * (1.0 + 1e-6), nq = sqrt(t[6]) * (1.0 + 1e-6);
+      const double A = fmin(t[0], nd * R) + fmin(t[1], nb * Rd);
+      const double T = fmin(t[2], nb * R);
+      const double Cs = fmin(t[3], nq * (R + Rd));
+      const size_t last = (size_t)cb * a.kcp + a.kcp - 1;
+      bool ok = true;
+      if (a.cand_id[last] >= 0 && kk > 0) {   // a list shorter than kc holds every allowed row
+        const double u = 1.0 / 16777216.0;
+        const int E = a.f32rows ? 4 : 8;
+        const double L = (double)E * ((a.dim + 32 * E - 1) / (32 * E));
+        const double slack = A + 2.0 * a.dim * u * T + (L + 5.0) * u * Cs;
+        const double wmax = a.weight_mode == ICD_WEIGHT_PRE ? 1.2 : 1.0;
+        const double s_kc = a.cand_score[last], kth = t_key[kk - 1];
+        ok = kth > s_kc + wmax * slack + 4.0 * u * (fabs(s_kc) + fabs(kth));
+      }
+      s_certified = ok ? 1 : 0;
+      if (!ok) {
+        a.fb[2 + atomicAdd(&a.fb[0], 1)] = b;
+        atomicAdd(&a.fb[1], 1);
+      }
+    }
+    __syncthreads();
+    if (!s_certified) return;
+  }
 
   // 3. reference re-rank: stable sort of the k hits by weighted score, descending
   for (int j = threadIdx.x; j < a.k; j += kFinThreads) {
@@ -314,7 +385,86 @@ __global__ void bf16_to_f32_kernel(const __nv_bfloat16* __restrict__ in, float* 
     out[i] = __bfloat162float(in[i]);
 }
 
+// per-column maxima of |value| (bf16 image and master) and of |master - bf16(master)| over a block of rows, folded into
+// colstat with integer atomicMax (non-negative floats order like their bit patterns)
+constexpr int kStatThreads = 256;
+__global__ void __launch_bounds__(kStatThreads)
+column_stats_kernel(const __nv_bfloat16* __restrict__ t, const float* __restrict__ m, int64_t n, int dim,
+                    float* __restrict__ colstat) {
+  constexpr int kCols = 1024 / kStatThreads;
+  __shared__ double red[3][kStatThreads / 32];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  float mx[kCols], dl[kCols];
+#pragma unroll
+  for (int j = 0; j < kCols; ++j) mx[j] = dl[j] = 0.f;
+  double rmax = 0.0, dmax = 0.0;   // largest squared row norms (thread 0): max(|bf16 row|, |master row|), |master - bf16|
+  for (int64_t r = blockIdx.x; r < n; r += gridDim.x) {
+    double ss_t = 0.0, ss_m = 0.0, ss_d = 0.0;
+#pragma unroll
+    for (int j = 0; j < kCols; ++j) {
+      const int c = threadIdx.x + j * kStatThreads;
+      if (c < dim) {
+        const float tv = __bfloat162float(t[(size_t)r * dim + c]);
+        float av = fabsf(tv);
+        ss_t += (double)tv * tv;
+        if (m) {
+          const float mv = m[(size_t)r * dim + c];
+          av = fmaxf(av, fabsf(mv));
+          dl[j] = fmaxf(dl[j], fabsf(mv - tv));
+          ss_m += (double)mv * mv;
+          ss_d += (double)(mv - tv) * (mv - tv);
+        }
+        mx[j] = fmaxf(mx[j], av);
+      }
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+      ss_t += __shfl_xor_sync(0xffffffffu, ss_t, off);
+      ss_m += __shfl_xor_sync(0xffffffffu, ss_m, off);
+      ss_d += __shfl_xor_sync(0xffffffffu, ss_d, off);
+    }
+    if (lane == 0) red[0][warp] = ss_t, red[1][warp] = ss_m, red[2][warp] = ss_d;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      double a0 = 0.0, a1 = 0.0, a2 = 0.0;
+      for (int w = 0; w < kStatThreads / 32; ++w) a0 += red[0][w], a1 += red[1][w], a2 += red[2][w];
+      rmax = fmax(rmax, fmax(a0, a1));
+      dmax = fmax(dmax, a2);
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    // rounded up: the norms enter an upper bound
+    atomicMax(reinterpret_cast<int*>(colstat) + 2 * dim, __float_as_int(__double2float_ru(sqrt(rmax) * (1.0 + 1e-6))));
+    atomicMax(reinterpret_cast<int*>(colstat) + 2 * dim + 1, __float_as_int(__double2float_ru(sqrt(dmax) * (1.0 + 1e-6))));
+  }
+#pragma unroll
+  for (int j = 0; j < kCols; ++j) {
+    const int c = threadIdx.x + j * kStatThreads;
+    if (c < dim) {
+      atomicMax(reinterpret_cast<int*>(colstat) + c, __float_as_int(mx[j]));
+      atomicMax(reinterpret_cast<int*>(colstat) + dim + c, __float_as_int(dl[j]));
+    }
+  }
+}
+
 }  // namespace
+
+int launch_column_stats(const void* table_bf16, const float* master, int64_t row0, int64_t n, int dim, float* colstat,
+                        cudaStream_t st) {
+  if (n <= 0) return ICD_OK;
+  if (dim > 1024) {
+    set_error("column_stats: dim %d > 1024", dim);
+    return ICD_E_ARG;
+  }
+  const int grid = (int)std::min<int64_t>(n, (int64_t)kSMs * 8);
+  column_stats_kernel<<<grid, kStatThreads, 0, st>>>(
+      reinterpret_cast<const __nv_bfloat16*>(table_bf16) + (size_t)row0 * dim, master ? master + (size_t)row0 * dim : nullptr,
+      n, dim, colstat);
+  count_launch();
+  ICD_CUDA(cudaGetLastError());
+  return ICD_OK;
+}
 
 int launch_merge(const MergeArgs& a, cudaStream_t st) {
   if (a.P > kMaxP || a.k_in > 255) {
@@ -323,7 +473,7 @@ int launch_merge(const MergeArgs& a, cudaStream_t st) {
   }
   const int grid = (a.B + kMergeWarps - 1) / kMergeWarps;
   merge_kernel<<<grid, kMergeWarps * 32, 0, st>>>(a.part_score, a.part_id, a.B, a.P, a.k_in, a.k_out,
-                                                 a.out_score, a.out_id, a.row_offset, a.bound_key_out);
+                                                 a.out_score, a.out_id, a.row_offset, a.bound_key_out, a.count);
   count_launch();
   ICD_CUDA(cudaGetLastError());
   return ICD_OK;

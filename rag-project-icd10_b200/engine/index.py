@@ -109,6 +109,14 @@ class VectorIndex:
                                                       1 if sync else 0), "icd_index_search")
         return score, raw, ids
 
+    def take_fallbacks(self) -> int:
+        """Queries the tensor path re-searched with the exact stream scan since the previous call (DESIGN.md, "Exact
+        search"); waits for the device."""
+        n = C.c_int64()
+        with self._lock:
+            N.check(N.lib().icd_index_take_fallbacks(self._h, C.byref(n)), "icd_index_take_fallbacks")
+        return int(n.value)
+
     def set_timing(self, on: bool) -> None:
         N.check(N.lib().icd_index_set_timing(self._h, 1 if on else 0), "icd_index_set_timing")
 
