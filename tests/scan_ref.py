@@ -121,9 +121,11 @@ def _check_order(ids, raw, score, levels, weight_mode):
 
 
 def certify(ids, raw, score, rows, q, k, weight_mode, levels, mask=None, f32rows=False, ref=None, strict=True,
-            top_outside=32):
+            top_outside=32, chunk_rows=None):
     """The exact-search rule.  ids/raw/score: [B, k] results; rows: what the index holds; q: the fp32 queries;
     levels: [n] uint8; mask: [n] bool of the allowed rows (None = all); ref: reference(rows, q, f32rows) to reuse.
+    chunk_rows: build the rules' summary (summarise) over row chunks of this size in fp64 instead of from the whole
+    [B, n] score matrix, so that tables of millions of rows certify in bounded memory; the verdict is the same.
 
     Structural rules (AssertionError whatever `strict`): count min(k, allowed), unique, allowed, -inf / -1 tail,
     order (raw desc, id asc), or (raw * w desc, id asc) with WEIGHT_PRE, or the stable re-rank by
@@ -131,9 +133,14 @@ def certify(ids, raw, score, rows, q, k, weight_mode, levels, mask=None, f32rows
     with a returned one must have the larger id.
     Bounded rules: |raw - exact| <= canonical bound per returned id; no allowed outside row beats a returned row by
     more than the two rows' combined bounds.  strict: AssertionError when either ratio exceeds 1."""
-    e, d = reference(rows, q, f32rows) if ref is None else ref
-    dev = e.device
-    B, n = e.shape
+    if chunk_rows is None:
+        e, d = reference(rows, q, f32rows) if ref is None else ref
+        dev, n = e.device, e.shape[1]
+        chunks = [(0, e, d)]
+    else:
+        dev, n = _t(q).device, rows.shape[0]
+        chunks = ((r0, *reference(rows[r0:r0 + chunk_rows], q, f32rows)) for r0 in range(0, n, chunk_rows))
+    B = q.shape[0]
     ids_t = _t(ids, dev, torch.int64)
     raw_t = _t(raw, dev, torch.float64)
     assert ids_t.shape == (B, k), (tuple(ids_t.shape), (B, k))
@@ -159,35 +166,19 @@ def certify(ids, raw, score, rows, q, k, weight_mode, levels, mask=None, f32rows
     assert bool(allowed[sel_ids].all()), "a masked-out row was returned"
     _check_order(ids_h, raw_h, score_h, lv_h, weight_mode)
 
+    s = summarise(sel_ids, chunks, weight_mode, levels, allowed, top_outside)
     # |raw - exact| per returned id
-    er = e.gather(1, sel_ids)
-    dr = d.gather(1, sel_ids)
-    score_ratio = float(((raw_t[:, :want] - er).abs() / dr.clamp_min(1e-300)).max())
-
-    # selection key and its bound
-    if weight_mode == WEIGHT_PRE:
-        w = weights_of(levels, dev)[None, :]
-        key = e * w
-        dk = d * w + 2 * U * key.abs()        # + the fp32 rounding of raw * w
-    else:
-        key, dk = e, d
-    inside = torch.zeros((B, n), dtype=torch.bool, device=dev)
-    inside.scatter_(1, sel_ids, True)
-    outside = allowed[None, :] & ~inside
+    score_ratio = float(((raw_t[:, :want] - s["er"]).abs() / s["dr"].clamp_min(1e-300)).max())
     gap_ratio = 0.0
     if n_allowed > want:
-        kj, dj = key.gather(1, sel_ids), dk.gather(1, sel_ids)
-        lo = (key - dk).masked_fill(~outside, -math.inf)
-        T = min(top_outside, n)
-        top_v, top_i = lo.topk(T, dim=1)
-        kr, drr = key.gather(1, top_i), dk.gather(1, top_i)
+        kj, dj, kr, drr, top_v, top_i = s["kj"], s["dj"], s["key"], s["dk"], s["lo"], s["id"]
         live = torch.isfinite(top_v)
         # pairwise (outside r, returned j)
         diff = kr[:, :, None] - kj[:, None, :]
         ratio = (diff / (drr[:, :, None] + dj[:, None, :]).clamp_min(1e-300)).masked_fill(~live[:, :, None], -math.inf)
         gap_ratio = max(0.0, float(ratio.max()))
         # the separable form of the same rule: max_r (key_r - dk_r) <= min_j (key_j + dk_j)
-        sep = (lo.max(1).values - (kj + dj).min(1).values)
+        sep = (top_v[:, 0] - (kj + dj).min(1).values)
         if bool((sep > 0).any()):
             gap_ratio = max(gap_ratio, 1.0 + 1e-12)
         # an exact tie broken the wrong way: an outside row with the same exact key and a lower id
@@ -199,6 +190,42 @@ def certify(ids, raw, score, rows, q, k, weight_mode, levels, mask=None, f32rows
         assert cert.score_ratio <= 1.0, f"returned raw scores off the exact ones by {cert.score_ratio:.3g}x the bound"
         assert cert.gap_ratio <= 1.0, f"an allowed row left out beats a returned one by {cert.gap_ratio:.3g}x the bound"
     return cert
+
+
+def summarise(sel_ids, chunks, weight_mode, levels, allowed, top_outside=32):
+    """The compact summary certify's bounded rules run on, accumulated over (row0, exact [B, m], bound [B, m]) chunks:
+    er / dr, the exact score and bound of each returned id; kj / dj, its selection key and key bound; and the running
+    top `top_outside` allowed rows outside the result by key - bound (lo), with their key, key bound and id."""
+    dev = sel_ids.device
+    B, want = sel_ids.shape
+    w_all = weights_of(levels, dev) if weight_mode == WEIGHT_PRE else None
+    z = torch.zeros((B, want), dtype=torch.float64, device=dev)
+    out = {"er": z, "dr": z, "kj": z, "dj": z}
+    top = [torch.empty((B, 0), dtype=torch.float64, device=dev) for _ in range(3)] + \
+          [torch.empty((B, 0), dtype=torch.int64, device=dev)]
+    for r0, e, d in chunks:
+        e, d = e.to(dev), d.to(dev)
+        m = e.shape[1]
+        if weight_mode == WEIGHT_PRE:
+            w = w_all[r0:r0 + m][None, :]
+            key = e * w
+            dk = d * w + 2 * U * key.abs()        # + the fp32 rounding of raw * w
+        else:
+            key, dk = e, d
+        loc = sel_ids - r0
+        here = (loc >= 0) & (loc < m)
+        locc = loc.clamp(0, m - 1)
+        for name, src in (("er", e), ("dr", d), ("kj", key), ("dj", dk)):
+            out[name] = torch.where(here, src.gather(1, locc), out[name])
+        inside = torch.zeros((B, m), dtype=torch.int32, device=dev).scatter_add_(1, locc, here.int()) > 0
+        lo = (key - dk).masked_fill(~(allowed[None, r0:r0 + m] & ~inside), -math.inf)
+        v, i = lo.topk(min(top_outside, m), dim=1)
+        cand = [torch.cat([top[0], v], 1), torch.cat([top[1], key.gather(1, i)], 1),
+                torch.cat([top[2], dk.gather(1, i)], 1), torch.cat([top[3], i + r0], 1)]
+        v, j = cand[0].topk(min(top_outside, cand[0].shape[1]), dim=1)
+        top = [v] + [c.gather(1, j) for c in cand[1:]]
+    out.update(lo=top[0], key=top[1], dk=top[2], id=top[3])
+    return out
 
 
 # ------------------------------------------------------------------------------------------------ probe corpora
@@ -252,3 +279,121 @@ def probe_corpus(n, dim, B, seed, spare_rows=()):
         rows[r] = row
         plants[l] = r
     return rows.astype(np.float32), q.astype(np.float32), plants
+
+
+# ------------------------------------------------------------------------------------------------ scan-side premises
+# The certificate of finalise_kernel (DESIGN.md, "Exact search") rests on three properties of the tensor scan's own
+# scores, checked one launch at a time by tests/test_scan_kernels_gpu.py:
+#   (a) the merged list is the top kc by scan score;
+#   (b) the pruning bound never exceeds the kc-th scan score (the pre-pass sees the main pass's bits);
+#   (c) a scan score is within A + T of the exact score.
+# These helpers give the bounds and the pre-pass model those tests compare against.
+TILE = 128             # rows per accumulator tile (MMA N) of the tensor scan
+PRE_SLOTS, PRE_FOLDS = 32, 4
+MIN_KEY = -2139062144  # 0x80808080 as int32: the very negative key of an empty bound
+
+
+def tc_term(dim):
+    """Factor of sum |bf16(q)_i * bf16(c)_i| that bounds the tensor core's fp32 accumulation (DESIGN.md: 2 dim 2^-24)."""
+    return 2.0 * dim * U
+
+
+def scan_bound(q, rows):
+    """Bound [B, n] of |tensor-scan score - exact q . rows| per (query, row), in the certificate's own terms.  The scan
+    multiplies bf16(q) with bf16(rows) on the tensor cores: T = 2 dim 2^-24 sum |bf16 q_i bf16 c_i|, plus, where the
+    query or the rows are not bf16 values, the exact input-rounding terms sum |q_i - bf16 q_i| |c_i| and
+    sum |bf16 q_i| |c_i - bf16 c_i| (both zero for bf16 inputs)."""
+    q = _t(q)
+    rows = _t(rows, q.device)
+    bq, bc = bf16_round(q.float()).double(), bf16_round(rows.float()).double()
+    bound = tc_term(q.shape[1]) * (bq.abs() @ bc.abs().T)
+    dq, dc = (q - bq).abs(), (rows - bc).abs()
+    if bool(dq.any()):
+        bound += dq @ rows.abs().T
+    if bool(dc.any()):
+        bound += bq.abs() @ dc.T
+    return bound
+
+
+def colstat_slack(q, colstat, f32rows):
+    """Per-query (A, T, C) of finalise_kernel's certificate in fp64, from a colstat [2 dim + 2] as launch_column_stats
+    leaves it: each term the smaller of its column-maxima form and its row-norm (Cauchy-Schwarz) form."""
+    q = _t(q)
+    cs = _t(colstat, q.device)
+    dim = q.shape[1]
+    M, D, Rn, Rd = cs[:dim], cs[dim:2 * dim], float(cs[2 * dim]), float(cs[2 * dim + 1])
+    bq = bf16_round(q.float()).double()
+    dq = q - bq
+    nd = dq.norm(dim=1) * (1 + 1e-6)
+    nb = bq.norm(dim=1) * (1 + 1e-6)
+    nq = q.norm(dim=1) * (1 + 1e-6)
+    A = torch.minimum(dq.abs() @ M, nd * Rn) + torch.minimum(bq.abs() @ D, nb * Rd)
+    T = tc_term(dim) * torch.minimum(bq.abs() @ M, nb * Rn)
+    L = lanes_fmas(dim, f32rows)
+    C = (L + 5) * U * torch.minimum(q.abs() @ (M + D), nq * (Rn + Rd))
+    return A, T, C
+
+
+def float_key(x):
+    """common.cuh float_key: the order-preserving int32 key of fp32 values (numpy)."""
+    i = np.ascontiguousarray(x, np.float32).view(np.int32)
+    return np.where(i >= 0, i, i ^ np.int32(0x7fffffff)).astype(np.int32)
+
+
+def sampled_tiles(n_rows, stride):
+    """Row tiles a pass at tile stride `stride` scans: tile index t' of the pass covers rows [t' s 128, t' s 128 + 128)."""
+    tiles = -(-n_rows // TILE)
+    return -(-tiles // max(1, stride))
+
+
+def tile_groups(n_tiles, G):
+    """Row group of each of the n_tiles tiles of a pass: group g owns tiles [n_tiles g / G, n_tiles (g + 1) / G)."""
+    g = np.arange(G)
+    owner = np.empty(n_tiles, np.int64)
+    for gi, (a, b) in enumerate(zip(n_tiles * g // G, n_tiles * (g + 1) // G)):
+        owner[a:b] = gi
+    return owner
+
+
+def slot_sets(n_rows, stride, G):
+    """The slot pre-pass's partition of the sampled rows: (rows, group, slot, class) for every sampled row r < n_rows;
+    slot = r mod 32 (the accumulator column mod 32), class = group mod 4 (bound_from_slots_kernel's fold)."""
+    nt = sampled_tiles(n_rows, stride)
+    owner = tile_groups(nt, G)
+    t = np.repeat(np.arange(nt), TILE)
+    col = np.tile(np.arange(TILE), nt)
+    rows = t * max(1, stride) * TILE + col
+    keep = rows < n_rows
+    rows, t, col = rows[keep], t[keep], col[keep]
+    g = owner[t]
+    return rows, g, col % PRE_SLOTS, g % PRE_FOLDS
+
+
+def expected_slot_max(scores, n_rows, stride, G, allowed=None):
+    """[B, G, 32] slot maxima the pre-pass must write, from the scores [B, n] (fp32, weights already applied) of every
+    row; masked-out rows and empty sets give -inf."""
+    s = np.asarray(scores, np.float32)
+    rows, g, slot, _ = slot_sets(n_rows, stride, G)
+    if allowed is not None:
+        keep = np.asarray(allowed, bool)[rows]
+        rows, g, slot = rows[keep], g[keep], slot[keep]
+    out = np.full((s.shape[0], G * PRE_SLOTS), -np.inf, np.float32)
+    idx = g * PRE_SLOTS + slot
+    for b in range(s.shape[0]):
+        np.maximum.at(out[b], idx, s[b, rows])
+    return out.reshape(s.shape[0], G, PRE_SLOTS)
+
+
+def bound_from_slots(slot_max, kc):
+    """Keys [B] of bound_from_slots_kernel: the slot maxima folded over the row groups of each class g mod 4, and the
+    kc-th largest of the 128 fold maxima (ties by fold index), or MIN_KEY when that is -inf."""
+    sm = np.asarray(slot_max, np.float32)
+    B, P, S = sm.shape
+    folds = np.full((B, PRE_FOLDS, S), -np.inf, np.float32)
+    for f in range(PRE_FOLDS):
+        if f < P:
+            folds[:, f] = sm[:, f::PRE_FOLDS].max(1)
+    v = folds.reshape(B, PRE_FOLDS * S)
+    o = np.lexsort((np.broadcast_to(np.arange(v.shape[1]), v.shape), -v.astype(np.float64)), axis=-1)
+    kth = np.take_along_axis(v, o[:, kc - 1:kc], 1)[:, 0]
+    return np.where(np.isneginf(kth), MIN_KEY, float_key(kth)).astype(np.int32)
