@@ -132,6 +132,27 @@ int icd_index_search(icd_index* idx, const void* q, int q_dtype, int B, int k, i
 int icd_index_search_filtered(icd_index* idx, const void* q, int q_dtype, int B, int k, int weight_mode, int path,
                               const uint32_t* row_mask, int64_t mask_rows, float* out_score, float* out_raw,
                               int64_t* out_id, void* stream, int sync);
+/* paged and range search beyond ICD_MAX_K (pymilvus's offset / limit and FLAT/IP range search).
+ * Let L be the list icd_index_search_filtered would return with k = offset + limit if k could be that large: the same
+ * canonical fp32 scores, (key desc, id asc) order, weight modes (ICD_WEIGHT_RERANK re-sorts the whole list of
+ * offset + limit raw hits) and mask rules -- after the range flags have removed every row whose RAW inner product lies
+ * outside (radius, range_filter] (Milvus's IP rule, in every weight mode).  The call writes L[offset, offset + limit)
+ * as [B, limit]; slots past the end of L are (-inf, -1).
+ *   page       offset >= 0, limit >= 1, offset + limit <= ICD_MAX_LIMIT; with both range flags radius < range_filter
+ * row_mask / mask_rows as icd_index_search_filtered; buffers, stream and sync as icd_index_search.  Every workspace
+ * size is known on the host, so the call enqueues without synchronising.  Exact by construction: every allowed row is
+ * scored, then a radix select and a sort (DESIGN.md, "Paged search"); a [chunk, n] fp32 workspace (<= 512 MiB)
+ * bounds the queries per pass. */
+#define ICD_MAX_LIMIT 16384  /* offset + limit, as pymilvus */
+#define ICD_RANGE_RADIUS 1   /* keep raw >  radius       */
+#define ICD_RANGE_FILTER 2   /* keep raw <= range_filter */
+typedef struct icd_search_page {
+  int32_t offset, limit, range_flags;
+  float radius, range_filter;
+} icd_search_page;
+int icd_index_search_page(icd_index* idx, const void* q, int q_dtype, int B, const icd_search_page* page,
+                          int weight_mode, const uint32_t* row_mask, int64_t mask_rows, float* out_score,
+                          float* out_raw, int64_t* out_id, void* stream, int sync);
 /* kernels launched / microseconds of device time of the last search on this handle, split by
  * stage: [0] scan, [1] merge, [2] rescore+finalise.  For bench.py's roofline line. */
 int icd_index_last_timing(const icd_index* idx, float* us3, int* launches);

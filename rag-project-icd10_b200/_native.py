@@ -22,6 +22,8 @@ WEIGHT_RERANK, WEIGHT_PRE, WEIGHT_NONE = 0, 1, 2
 PATH_AUTO, PATH_STREAM, PATH_TENSOR = 0, 1, 2
 INDEX_KEEP_F32 = 1
 MAX_K = 128
+MAX_LIMIT = 16384          # offset + limit of icd_index_search_page, as pymilvus
+RANGE_RADIUS, RANGE_FILTER = 1, 2
 
 # every symbol include/icdrag.h declares (tests check the library exports each one)
 SYMBOLS = [
@@ -29,6 +31,7 @@ SYMBOLS = [
     "icd_index_create", "icd_index_destroy", "icd_index_append", "icd_index_adopt", "icd_index_clear",
     "icd_index_size", "icd_index_dim", "icd_index_read", "icd_index_search", "icd_index_last_timing",
     "icd_index_set_timing", "icd_index_mean_timing", "icd_index_search_filtered", "icd_index_take_fallbacks",
+    "icd_index_search_page",
     "icd_nccl_unique_id", "icd_shard_group_create", "icd_shard_group_destroy",
     "icd_shard_group_export_slab", "icd_shard_group_import_slabs", "icd_shard_group_search",
     "icd_shard_group_search_filtered",
@@ -48,6 +51,13 @@ class BertCfg(C.Structure):
     _fields_ = [("vocab_size", C.c_int32), ("hidden", C.c_int32), ("layers", C.c_int32),
                 ("heads", C.c_int32), ("intermediate", C.c_int32), ("max_position", C.c_int32),
                 ("type_vocab", C.c_int32), ("ln_eps", C.c_float)]
+
+
+class SearchPage(C.Structure):
+    """icd_search_page: the page [offset, offset + limit) of the exact list, after the range (radius, range_filter]
+    on the raw inner product (range_flags = RANGE_RADIUS | RANGE_FILTER)."""
+    _fields_ = [("offset", C.c_int32), ("limit", C.c_int32), ("range_flags", C.c_int32),
+                ("radius", C.c_float), ("range_filter", C.c_float)]
 
 
 _lib = None
@@ -116,6 +126,7 @@ def _declare(L: C.CDLL) -> None:
     L.icd_index_set_timing.argtypes = [vp, i32]
     L.icd_index_mean_timing.argtypes = [vp, f32p, C.POINTER(i32)]
     L.icd_index_take_fallbacks.argtypes = [vp, C.POINTER(i64)]
+    L.icd_index_search_page.argtypes = [vp, vp, i32, i32, C.POINTER(SearchPage), i32, vp, i64, vp, vp, vp, vp, i32]
     if hasattr(L, "icd_nccl_unique_id"):
         L.icd_nccl_unique_id.argtypes = [vp]
         L.icd_shard_group_create.argtypes = [vp, i32, i32, i64, vp, C.POINTER(vp)]

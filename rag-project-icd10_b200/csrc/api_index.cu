@@ -455,6 +455,7 @@ int icd_index_destroy(icd_index* x) {
   x->q_f32_alt.release();
   x->q_bf16_alt.release();
   x->out_stage_alt.release();
+  x->page_ws.release();
   if (x->copy_stream) cudaStreamDestroy(x->copy_stream);
   for (int i = 0; i < 2; ++i) {
     if (x->ev_ready[i]) cudaEventDestroy(x->ev_ready[i]);
@@ -731,6 +732,79 @@ int icd_index_search_filtered(icd_index* x, const void* q, int q_dtype, int B, i
     ICD_TRY(copy_out(o_score, k_score, (size_t)nb * k * 4, st));
     ICD_TRY(copy_out(o_raw, k_raw, (size_t)nb * k * 4, st));
     ICD_TRY(copy_out(o_id, k_id, (size_t)nb * k * 8, st));
+    if (B > kMaxBatch) ICD_CUDA(cudaStreamSynchronize(st));  // staging buffers are reused
+  }
+  if (sync || host_out || !is_device_ptr(q)) ICD_CUDA(cudaStreamSynchronize(st));
+  return ICD_OK;
+}
+
+int icd_index_search_page(icd_index* x, const void* q, int q_dtype, int B, const icd_search_page* page, int weight_mode,
+                          const uint32_t* row_mask, int64_t mask_rows, float* out_score, float* out_raw, int64_t* out_id,
+                          void* stream, int sync) {
+  ICD_CHECK_ARG(x != nullptr, "index is null");
+  ICD_CHECK_ARG(page != nullptr, "page is null");
+  ICD_CHECK_ARG(B >= 0, "negative batch");
+  ICD_CHECK_ARG(page->limit >= 1, "limit must be >= 1");
+  ICD_CHECK_ARG(page->offset >= 0, "offset must be >= 0");
+  ICD_CHECK_ARG((int64_t)page->offset + page->limit <= ICD_MAX_LIMIT, "offset + limit must be <= 16384");
+  ICD_CHECK_ARG((page->range_flags & ~(ICD_RANGE_RADIUS | ICD_RANGE_FILTER)) == 0, "unknown range flags");
+  ICD_CHECK_ARG(page->range_flags != (ICD_RANGE_RADIUS | ICD_RANGE_FILTER) || page->radius < page->range_filter,
+                "radius must be below range_filter");
+  ICD_CHECK_ARG(weight_mode >= 0 && weight_mode <= 2, "unknown weight mode");
+  if (row_mask && mask_rows != x->n) {
+    set_error("row mask covers %lld rows, the table holds %lld", (long long)mask_rows, (long long)x->n);
+    return ICD_E_ARG;
+  }
+  if (B == 0) return ICD_OK;
+  ICD_CHECK_ARG(q != nullptr, "q is null");
+  DeviceGuard g(x->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int limit = page->limit, K = page->offset + page->limit;
+  const bool host_out = (out_score && !is_device_ptr(out_score)) || (out_raw && !is_device_ptr(out_raw)) ||
+                        (out_id && !is_device_ptr(out_id));
+  const uint32_t* d_mask = nullptr;
+  ICD_TRY(index_stage_mask(x, row_mask, mask_rows, &d_mask, st));
+  constexpr int kMaxBatch = 8192;  // bounds the query staging; larger batches run as several passes
+  const int chunk = page_search_chunk(x->n, K, std::min(B, kMaxBatch));
+  const size_t ws_bytes = page_search_workspace_bytes(x->n, K, chunk);
+  ICD_TRY(x->page_ws.reserve(ws_bytes));
+  for (int b0 = 0; b0 < B; b0 += kMaxBatch) {
+    const int nb = std::min(kMaxBatch, B - b0);
+    const size_t qoff = (size_t)b0 * x->dim * (q_dtype == ICD_F32 ? 4 : 2);
+    ICD_TRY(index_stage_queries(x, (const char*)q + qoff, q_dtype, nb, st));
+    // device-side result buffers: caller's when on device, staging otherwise
+    ICD_TRY(x->out_stage.reserve((size_t)nb * limit * 16));
+    float* d_score = (float*)x->out_stage.ptr;
+    float* d_raw = d_score + (size_t)nb * limit;
+    int64_t* d_id = (int64_t*)(d_raw + (size_t)nb * limit);
+    float* o_score = out_score ? out_score + (size_t)b0 * limit : nullptr;
+    float* o_raw = out_raw ? out_raw + (size_t)b0 * limit : nullptr;
+    int64_t* o_id = out_id ? out_id + (size_t)b0 * limit : nullptr;
+    PageSearchArgs a{};
+    a.rows = x->master ? (const void*)x->master : (const void*)x->table;
+    a.f32rows = x->master != nullptr;
+    a.levels = x->levels;
+    a.n = x->n;
+    a.dim = x->dim;
+    a.q = (const float*)x->q_f32.ptr;
+    a.nq = nb;
+    a.mask = d_mask;
+    a.range_flags = page->range_flags;
+    a.radius = page->radius;
+    a.range_filter = page->range_filter;
+    a.weight_mode = weight_mode;
+    a.offset = page->offset;
+    a.limit = limit;
+    a.chunk = chunk;
+    a.workspace = x->page_ws.ptr;
+    a.workspace_bytes = x->page_ws.cap;
+    a.out_score = (o_score && is_device_ptr(o_score)) ? o_score : (o_score ? d_score : nullptr);
+    a.out_raw = (o_raw && is_device_ptr(o_raw)) ? o_raw : (o_raw ? d_raw : nullptr);
+    a.out_id = (o_id && is_device_ptr(o_id)) ? o_id : (o_id ? d_id : nullptr);
+    ICD_TRY(launch_page_search(a, st));
+    ICD_TRY(copy_out(o_score, a.out_score, (size_t)nb * limit * 4, st));
+    ICD_TRY(copy_out(o_raw, a.out_raw, (size_t)nb * limit * 4, st));
+    ICD_TRY(copy_out(o_id, a.out_id, (size_t)nb * limit * 8, st));
     if (B > kMaxBatch) ICD_CUDA(cudaStreamSynchronize(st));  // staging buffers are reused
   }
   if (sync || host_out || !is_device_ptr(q)) ICD_CUDA(cudaStreamSynchronize(st));

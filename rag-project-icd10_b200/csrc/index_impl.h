@@ -50,6 +50,7 @@ struct icd_index {
   int64_t timed_calls = 0;   // searches recorded since timing was switched on
   bool timing = false, timing_pending = false;
   int last_launches = 0;
+  icd::DeviceBuf page_ws;   // icd_index_search_page: [chunk, n] scores, select state, gathered lists (topk_large.cu)
 };
 
 namespace icd {

@@ -136,6 +136,32 @@ struct FinaliseArgs {
 };
 int launch_finalise(const FinaliseArgs& a, cudaStream_t st);
 
+// ---- topk_large.cu: exact paged search, K = offset + limit <= ICD_MAX_LIMIT (icd_index_search_page)
+struct PageSearchArgs {
+  const void* rows;       // [n, dim] bf16 table or fp32 master (f32rows): the rows finalise_kernel rescores
+  bool f32rows;
+  const uint8_t* levels;  // [n]
+  int64_t n;
+  int dim;
+  const float* q;         // [nq, dim] fp32 device
+  int nq;
+  const uint32_t* mask;   // row bitmap, null = every row
+  int range_flags;        // ICD_RANGE_RADIUS | ICD_RANGE_FILTER, on the raw inner product
+  float radius, range_filter;
+  int weight_mode;
+  int offset, limit;
+  int chunk;              // queries per workspace pass (page_search_chunk)
+  void* workspace;        // page_search_workspace_bytes(n, offset + limit, chunk) device bytes
+  size_t workspace_bytes;
+  float* out_score;       // [nq, limit] device, each may be null
+  float* out_raw;
+  int64_t* out_id;
+};
+// queries per pass for a batch of B: the [chunk, n] fp32 score workspace stays within a fixed budget (512 MiB)
+int page_search_chunk(int64_t n, int K, int B);
+size_t page_search_workspace_bytes(int64_t n, int K, int chunk);
+int launch_page_search(const PageSearchArgs& a, cudaStream_t st);
+
 // elementwise helpers
 int launch_f32_to_bf16(const float* in, void* out_bf16, int64_t n, cudaStream_t st);
 int launch_bf16_to_f32(const void* in_bf16, float* out, int64_t n, cudaStream_t st);

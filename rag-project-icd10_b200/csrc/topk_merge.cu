@@ -4,6 +4,7 @@
 //   finalise_kernel  candidates -> exact fp32 rescoring -> sort -> cut to k -> the reference's
 //                    level weighting and re-sort (services/milvus_service.py:290-314,550-558)
 // Both are latency-sized (k <= 128 candidates per list); the roofline kernel is the scan.
+#include "canon_dot.cuh"
 #include "common.cuh"
 #include "kernels.h"
 
@@ -110,38 +111,6 @@ bound_from_slots_kernel(const float* __restrict__ slot_max, int B, int P, int kc
     rank += (v > m || (v == m && o < (int)threadIdx.x)) ? 1 : 0;
   }
   if (rank == kc - 1) bound_key_out[b] = (m == -INFINITY) ? (int)0x80808080 : float_key(m);
-}
-
-// canonical exact dot: chunk c of the row belongs to lane c%32, chunks ascending, elements
-// ascending, then xor-butterfly -- identical to scan_stream.cu
-template <bool F32ROWS>
-__device__ __forceinline__ float warp_dot_row(const void* rows, int64_t row, int dim, const float* q, int lane) {
-  constexpr int E = F32ROWS ? 4 : 8;
-  const int nchunks = dim / E;
-  const char* base = reinterpret_cast<const char*>(rows) + (size_t)row * dim * (F32ROWS ? 4 : 2);
-  float acc = 0.f;
-  for (int c = lane; c < nchunks; c += 32) {
-    const uint4 v = *reinterpret_cast<const uint4*>(base + (size_t)c * 16);
-    const float* qs = q + c * E;
-    if constexpr (F32ROWS) {
-      acc = fmaf(__uint_as_float(v.x), qs[0], acc);
-      acc = fmaf(__uint_as_float(v.y), qs[1], acc);
-      acc = fmaf(__uint_as_float(v.z), qs[2], acc);
-      acc = fmaf(__uint_as_float(v.w), qs[3], acc);
-    } else {
-      acc = fmaf(bf16lo_to_f32(v.x), qs[0], acc);
-      acc = fmaf(bf16hi_to_f32(v.x), qs[1], acc);
-      acc = fmaf(bf16lo_to_f32(v.y), qs[2], acc);
-      acc = fmaf(bf16hi_to_f32(v.y), qs[3], acc);
-      acc = fmaf(bf16lo_to_f32(v.z), qs[4], acc);
-      acc = fmaf(bf16hi_to_f32(v.z), qs[5], acc);
-      acc = fmaf(bf16lo_to_f32(v.w), qs[6], acc);
-      acc = fmaf(bf16hi_to_f32(v.w), qs[7], acc);
-    }
-  }
-#pragma unroll
-  for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
-  return acc;
 }
 
 constexpr int kFinThreads = 256;

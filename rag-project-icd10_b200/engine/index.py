@@ -77,13 +77,18 @@ class VectorIndex:
 
     # ---------------------------------------------------------------- search
     def search(self, q, k: int, weight_mode: int = N.WEIGHT_RERANK, path: int = N.PATH_AUTO,
-               out: Optional[Tuple] = None, stream: int = 0, sync: bool = True, mask=None):
+               out: Optional[Tuple] = None, stream: int = 0, sync: bool = True, mask=None, offset: int = 0,
+               radius: Optional[float] = None, range_filter: Optional[float] = None):
         """q: [B, dim] float32/bfloat16, numpy (host) or torch (host/device).
 
         Returns (score [B,k] f32, raw [B,k] f32, ids [B,k] i64) in the memory space of q
         (numpy for numpy, torch tensors on q's device for torch), or fills `out`.
         mask: packed uint32 row bitmap (engine/filter_expr.py::pack_bits; numpy or a CUDA tensor): the exact top-k over
-        the rows whose bit is set; fewer than k such rows leave a (-inf, -1) tail.  None = every row."""
+        the rows whose bit is set; fewer than k such rows leave a (-inf, -1) tail.  None = every row.
+        offset / radius / range_filter (pymilvus's paging and FLAT/IP range search): the hits [offset, offset + k) of
+        the exact list over the rows whose raw inner product lies in (radius, range_filter]; offset + k <= MAX_LIMIT.
+        k <= MAX_K with no offset and no range is today's icd_index_search_filtered call; anything else is
+        icd_index_search_page, which has one exact path (path must be PATH_AUTO)."""
         if q.ndim == 1:
             q = q[None, :]
         B = int(q.shape[0])
@@ -101,6 +106,23 @@ class VectorIndex:
                 ids = np.empty((B, k), np.int64)
         else:
             score, raw, ids = out
+        paged = k > N.MAX_K or offset != 0 or radius is not None or range_filter is not None
+        if paged and path != N.PATH_AUTO:
+            raise ValueError("searches beyond k = 128, with an offset or with a range have one exact path: "
+                             "path must be PATH_AUTO")
+        if paged:
+            page = N.SearchPage(offset=int(offset), limit=int(k),
+                                range_flags=(N.RANGE_RADIUS if radius is not None else 0)
+                                | (N.RANGE_FILTER if range_filter is not None else 0),
+                                radius=float(radius) if radius is not None else 0.0,
+                                range_filter=float(range_filter) if range_filter is not None else 0.0)
+            with self._lock:
+                n = len(self)
+                N.check(N.lib().icd_index_search_page(self._h, N.buf_ptr(q), N.vec_dtype(q), B, C.byref(page),
+                                                      int(weight_mode), N.mask_ptr(mask, n), n, N.buf_ptr(score),
+                                                      N.buf_ptr(raw), N.buf_ptr(ids), C.c_void_p(stream),
+                                                      1 if sync else 0), "icd_index_search_page")
+            return score, raw, ids
         with self._lock:
             n = len(self)
             N.check(N.lib().icd_index_search_filtered(self._h, N.buf_ptr(q), N.vec_dtype(q), B, int(k), int(weight_mode),

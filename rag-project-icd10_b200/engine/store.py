@@ -685,24 +685,63 @@ class IcdStoreClient:
             self._masks.popitem(last=False)
         return dev
 
+    @staticmethod
+    def _page(limit, search_params=None, offset=None):
+        """pymilvus's paging and range arguments -> (limit, offset, radius, range_filter), checked by pymilvus's rules:
+        1 <= limit, 0 <= offset, offset + limit <= 16 384; offset given as `offset=` or search_params["offset"] (both
+        only when equal); radius / range_filter from search_params["params"] (FLAT/IP range search: the hits whose
+        inner product lies in (radius, range_filter]), radius < range_filter when both are given."""
+        sp = search_params or {}
+        if not isinstance(sp, dict):
+            raise ValueError(f"search_params must be a dict, got {type(sp).__name__}")
+        sp_offset = sp.get("offset")
+        if offset is not None and sp_offset is not None and int(offset) != int(sp_offset):
+            raise ValueError(f"conflicting offsets: offset={offset} and search_params['offset']={sp_offset}")
+        offset = int(offset if offset is not None else (sp_offset or 0))
+        limit = int(limit)
+        if limit < 1:
+            raise ValueError(f"limit must be >= 1, got {limit}")
+        if offset < 0:
+            raise ValueError(f"offset must be >= 0, got {offset}")
+        if offset + limit > N.MAX_LIMIT:
+            raise ValueError(f"offset + limit must be in [1, {N.MAX_LIMIT}], got {offset} + {limit}")
+        params = sp.get("params") or {}
+        radius, range_filter = params.get("radius"), params.get("range_filter")
+        radius = None if radius is None else float(radius)
+        range_filter = None if range_filter is None else float(range_filter)
+        if radius is not None and range_filter is not None and not radius < range_filter:
+            raise ValueError(f"range search on IP needs radius < range_filter, got {radius} and {range_filter}")
+        return limit, offset, radius, range_filter
+
+    @staticmethod
+    def _group_refuses(limit, offset, radius, range_filter) -> None:
+        if limit > N.MAX_K or offset or radius is not None or range_filter is not None:
+            raise NotImplementedError(f"a sharded collection serves limit <= {N.MAX_K} without offset or range "
+                                      "(paged and range search run on a single-table collection)")
+
     def search(self, collection_name: str, data, limit: int = 10, output_fields: Optional[List[str]] = None,
-               filter: str = "", **_kw) -> List[List[Hit]]:
+               filter: str = "", search_params: Optional[Dict[str, Any]] = None, offset: Optional[int] = None,
+               **_kw) -> List[List[Hit]]:
         """MilvusClient.search; `filter` = a boolean expression over the scalar fields (engine/filter_expr.py): the exact
-        top-`limit` over the rows it allows (fewer hits when fewer rows match).  ValueError on a bad expression."""
+        top-`limit` over the rows it allows (fewer hits when fewer rows match).  ValueError on a bad expression.
+        `offset` (or search_params["offset"]) skips the first hits, search_params["params"] may hold `radius` /
+        `range_filter` (range search on the raw inner product); offset + limit <= 16 384 (_page)."""
         col = self.cols[collection_name]
         if not col.loaded or col.index is None:
             raise N.NativeError(f"collection {collection_name} is not loaded")
+        k, offset, radius, range_filter = self._page(limit, search_params, offset)
         q = np.ascontiguousarray(np.asarray(data, dtype=np.float32))
         if q.ndim == 1:
             q = q[None, :]
-        k = max(1, min(int(limit), N.MAX_K))
         mask = self._row_mask(col, filter)
         group = getattr(col, "group", None)
         if group is not None:
+            self._group_refuses(k, offset, radius, range_filter)
             _, raw, ids = group.search(q, k, weight_mode=N.WEIGHT_NONE, mask=mask)
             base = 0
         else:
-            _, raw, ids = col.index.search(q, k, weight_mode=N.WEIGHT_NONE, mask=mask)
+            _, raw, ids = col.index.search(q, k, weight_mode=N.WEIGHT_NONE, mask=mask, offset=offset, radius=radius,
+                                           range_filter=range_filter)
             base = col.row_lo
         fields = output_fields or []
         out = []
@@ -721,18 +760,20 @@ class IcdStoreClient:
         """Batched search with the level re-rank done on the GPU (ICD_WEIGHT_RERANK: raw top-k, score x w(level),
         stable re-sort -- milvus_service.py:290-314): returns (score [B,k] f32, raw [B,k] f32, ids [B,k] i64 GLOBAL
         row ids, -1 = no hit) as numpy arrays; scalar fields are fetched lazily through row() / field().  `filter` as
-        in search()."""
+        in search(); limit <= 16 384."""
         col = self.cols[collection_name]
         if not col.loaded or col.index is None:
             raise N.NativeError(f"collection {collection_name} is not loaded")
+        k, _, _, _ = self._page(limit)
         q = np.ascontiguousarray(np.asarray(queries, dtype=np.float32))
         if q.ndim == 1:
             q = q[None, :]
         mask = self._row_mask(col, filter)
         group = getattr(col, "group", None)
         if group is not None:
-            return group.search(q, max(1, min(int(limit), N.MAX_K)), weight_mode=N.WEIGHT_RERANK, mask=mask)
-        score, raw, ids = col.index.search(q, max(1, min(int(limit), N.MAX_K)), weight_mode=N.WEIGHT_RERANK, mask=mask)
+            self._group_refuses(k, 0, None, None)
+            return group.search(q, k, weight_mode=N.WEIGHT_RERANK, mask=mask)
+        score, raw, ids = col.index.search(q, k, weight_mode=N.WEIGHT_RERANK, mask=mask)
         if col.row_lo:
             ids = np.where(ids >= 0, ids + col.row_lo, ids)
         return score, raw, ids
